@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Headline benchmark: spectra/sec for the full 60-alpha MaxEnt loop in FP64 (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (data projection -> fused alpha sweep -> analyzers) over one
 synthetic bootstrap batch: per GPU, `--spectra` (default 8192 = BASELINE config 5's per-GPU shard of the
@@ -53,6 +53,9 @@ def parse_args():
                     help="secondary measurements only: the headline metric is the default (normal) cost function")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-procs", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed to DIR/<name>.npy (float64, under 64 MB: "
+                         "a fixed, seeded sample of the spectra)")
     return ap.parse_args()
 
 
@@ -183,6 +186,34 @@ def algorithmic_flops(n_iter, n_q, n_s, n_alpha_total, n_omega, s, probability):
     if probability:
         F += n_alpha_total * (n_omega * s * s + s ** 3 / 3.0)
     return F
+
+
+DUMP_BYTES = 60 * 10 ** 6          # data of --dump-outputs: under 64 MB with the .npy headers
+DUMP_ANALYZERS = 3                 # LineFit, Chi2Curvature, Entropy: Classic and Bryan need the probability (not computed)
+
+
+def dump_outputs(res, out_dir):
+    """Write the result of one device-resident step (engine.SweepResult) to out_dir/<name>.npy in float64, so that two
+    builds can be compared output for output: ``alpha`` and, for a fixed seeded sample of the batch (``spectrum_index``,
+    as many spectra as fit in DUMP_BYTES), ``chi2``, ``S``, ``Q`` [n, n_alpha], ``alpha_index`` [n, 3], ``A_out``
+    [n, 3, n_omega] and ``A`` [n, n_alpha, n_omega].  The solver's counters (n_iter, status, ...) describe how a result
+    was reached rather than the result, and this path computes no probability (``logp``, Classic and Bryan analyzers):
+    neither is written.  In a multi-GPU job rank 0 writes its own shard."""
+    import numpy as np
+    import torch
+    B, n_alpha, n_omega = res.A.shape
+    n_an = DUMP_ANALYZERS
+    per_spectrum = 8 * (1 + 3 * n_alpha + n_an + n_an * n_omega + n_alpha * n_omega)
+    n = min(B, (DUMP_BYTES - 8 * n_alpha) // per_spectrum)
+    rows = np.sort(np.random.default_rng(0).choice(B, n, replace=False))
+    idx = torch.as_tensor(rows, device=res.A.device)
+    arrays = {"alpha": res.alpha, "spectrum_index": torch.as_tensor(rows), "alpha_index": res.alpha_index[idx, :n_an],
+              "A_out": res.A_out[idx, :n_an]}
+    for name in ("chi2", "S", "Q", "A"):
+        arrays[name] = getattr(res, name)[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.cpu().numpy().astype(np.float64))
 
 
 def run_native(a):
@@ -397,6 +428,8 @@ def run_native(a):
                          "frac_with_survey_formula": flops_survey / (kernel_ms * 1e-3) / 1e12 / peak,
                          "pipe": "FP64 (DMMA m8n8k4 + DFMA share one pipe on B200)", "peak_source": peak_src},
         }
+        if a.dump_outputs:
+            dump_outputs(res, a.dump_outputs)
         if world == 1 and not a.no_cpu_baseline and a.cost_function == "normal":
             try:
                 line["cpu_baseline"] = cpu_baseline_block(cpu_baseline(a))

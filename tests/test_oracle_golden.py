@@ -5,8 +5,20 @@ import os
 
 import numpy as np
 import pytest
+import threadpoolctl
 
 from oracle import maxent_oracle as mo
+
+# oracle/make_golden.py wrote the fixtures on a host whose OpenBLAS ran its SkylakeX (AVX-512) kernels on 8 threads.
+# How OpenBLAS splits a matrix product over its threads changes the last bits of the result, so the bit-identical
+# comparisons below run on that many BLAS threads, whatever the number of cores of the host running the tests.
+GOLDEN_BLAS_THREADS = 8
+
+
+@pytest.fixture(scope="module", autouse=True)
+def _golden_blas_threads():
+    with threadpoolctl.threadpool_limits(limits=GOLDEN_BLAS_THREADS, user_api="blas"):
+        yield
 
 
 def _load(golden_dir, name):

@@ -1,6 +1,6 @@
 import os, sys, json
-sys.path.insert(0, "/root/repo")
-os.environ["MAXENT_B200_LIB"] = "/root/repo/maxent_b200/libmaxent_b200_tprof.so"
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+os.environ["MAXENT_B200_LIB"] = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "maxent_b200/libmaxent_b200_tprof.so")
 import numpy as np, torch
 from maxent_b200 import batched, engine
 job = batched.BatchedTauMaxEnt(reduce_singular_space=1e-11)
