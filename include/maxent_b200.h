@@ -207,6 +207,20 @@ int mx_analyze(const double* alpha /*[n_alpha]*/, const double* chi2, const doub
                int32_t bryan_by_integration,
                int32_t* alpha_index, double* A_out, double* aux, void* stream);
 
+/* PoormanMaxEnt off-diagonal default models (python/elementwise_maxent.py:633-652) for P off-diagonal spectra, read from
+ * the analyzer output of the diagonal pass (A_out of mx_analyze, R spectra) without a trip to the host:
+ *   D[p]  = (sqrt(A_out[rows[2p], slot] * A_out[rows[2p+1], slot]) + d_add) * delta  (DataDefaultModel(...).D), rows of
+ *           ldD = n_omega rounded up to an even number, padding zeroed (the layout of MX_PER_SPECTRUM_MODEL);
+ *   v0[p] = V'^T log(arg), arg = (H0 + sqrt(H0^2 + 4 D^2)) / (2 D), H0 = (A_init or D[p]) * delta (maxent_loop.py:
+ *           196-203), |arg| <= 1e-100 -> 1e-100; V' = Vp + group[p] * n_omega * n_sv (Vp[G, n_omega, n_sv], group may
+ *           be NULL: G = 1).  Summed over omega in index order: independent of P and of p's position in the batch;
+ *   ok[p] = 0 when either diagonal row holds a NaN (analyzer unavailable, element not continued), else 1.
+ * The caller guarantees 0 <= rows < R and 0 <= group < G. */
+int mx_poorman_models(const double* A_out /*[R, MX_N_ANALYZERS, n_omega]*/, int32_t slot, const int32_t* rows /*[P, 2]*/,
+                      int32_t P, const double* delta, double d_add, const double* A_init /*[n_omega] or NULL*/,
+                      const double* Vp, const int32_t* group /*[P] or NULL*/, int32_t n_omega, int32_t n_sv,
+                      double* D /*[P, ldD]*/, double* v0 /*[P, n_sv]*/, int32_t* ok /*[P]*/, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -74,6 +74,8 @@ SYMBOLS = [
                                        ctypes.POINTER(ctypes.c_int32)]),
     ("mx_analyze", ctypes.c_int, [c_dp, c_dp, c_dp, c_dp, c_dp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                   ctypes.c_double, ctypes.c_int32, ctypes.c_int32, c_dp, c_dp, c_dp, c_dp]),
+    ("mx_poorman_models", ctypes.c_int, [c_dp, ctypes.c_int32, c_dp, ctypes.c_int32, c_dp, ctypes.c_double, c_dp, c_dp,
+                                         c_dp, ctypes.c_int32, ctypes.c_int32, c_dp, c_dp, c_dp, c_dp]),
 ]
 
 _lib = None

@@ -177,8 +177,16 @@ class BatchedTauMaxEnt(object):
         self.err = err
         self.cov = None
         self._per_spectrum = per_spectrum
+        self._groups = None
         self.problem = None
         self._group_cache = {}
+
+    def set_error_groups(self, err, index):
+        """Whitening groups given directly: ``err`` [G, n_tau] holds G error vectors and ``index`` [B] the group of every
+        spectrum -- the [B, n_tau] case of ``set_error`` without the copy per spectrum (the batched matrix front ends map
+        per-element error vectors to groups by element index)."""
+        self.set_error(np.asarray(err, dtype=np.float64))
+        self._groups = np.asarray(index, dtype=np.int64).reshape(-1)
 
     def set_cov(self, cov, cov_threshold=1.e-14):
         """Covariance matrix of the data, [n_tau, n_tau] shared by the batch or [B, n_tau, n_tau] per spectrum
@@ -189,6 +197,7 @@ class BatchedTauMaxEnt(object):
         self.cov = cov
         self.cov_threshold = cov_threshold
         self.err = None
+        self._groups = None
         self.problem = None
         self._group_cache = {}
 
@@ -214,6 +223,10 @@ class BatchedTauMaxEnt(object):
         if self.err is None:
             raise Exception("no error set: call set_error")
         err = np.asarray(self.err, dtype=np.float64)
+        if getattr(self, "_groups", None) is not None:
+            if self._groups.shape != (B,) or err.ndim != 2 or err.shape[1] != n_tau:
+                raise Exception("error groups: %s vectors for %d spectra, index %s" % (err.shape, B, self._groups.shape))
+            return "groups", self._groups, [(None, e) for e in err]
         if err.ndim == 0 or (err.ndim == 1 and err.shape[0] == n_tau and not self._per_spectrum):
             return "shared", None, None
         if err.ndim == 1:
@@ -293,9 +306,10 @@ class BatchedTauMaxEnt(object):
             return a * self.prepare().n_tau
         return a * float(self.scale_alpha)
 
-    def run_device(self, G_dev, want_A=True, want_v=False, D=None, skip_small=False):
+    def run_device(self, G_dev, want_A=True, want_v=False, D=None, skip_small=False, v0=None):
         """Hot path on device-resident data: returns an engine.SweepResult of device tensors.
-        ``D`` [B, n_omega] (optional): one default model per spectrum, incl. delta omega like ``DefaultModel.D``.
+        ``D`` [B, n_omega] (optional): one default model per spectrum, incl. delta omega like ``DefaultModel.D``; with
+        ``v0`` [B, n_sv] the model rows are ready-made (D [B, ldD], engine.run_sweep).
         Per-spectrum error models (set_error / set_cov with a leading batch axis) are applied here.
         ``skip_small``: spectra with max|G| < G_threshold are NOT continued (python/maxent_loop.py:174-179): they are left
         out of the launch and come back with status MX_STATUS_SKIPPED, NaN scalars, alpha_index -1 and A = 0."""
@@ -303,10 +317,11 @@ class BatchedTauMaxEnt(object):
         if skip_small and G_dev.dim() > 1 and G_dev.shape[0]:
             small = G_dev.abs().amax(dim=1) < self.G_threshold
             if bool(small.any()):
-                return self._run_without(G_dev, small, want_A, want_v, D)
+                return self._run_without(G_dev, small, want_A, want_v, D, v0)
         prob = self.prepare()
         kw = dict(probability=self.probability is not None, lm=self.minimizer, want_A=want_A, want_v=want_v,
-                  gamma=self.gamma, linefit_deg=self.linefit_deg, bryan_by_integration=self.bryan_by_integration, D=D)
+                  gamma=self.gamma, linefit_deg=self.linefit_deg, bryan_by_integration=self.bryan_by_integration, D=D,
+                  v0=v0)
         B = int(G_dev.shape[0]) if G_dev.dim() > 1 else 1
         mode, a, specs = self._error_plan(B)
         if mode == "shared":
@@ -336,7 +351,7 @@ class BatchedTauMaxEnt(object):
         res.alpha_scale = scale
         return res
 
-    def _run_without(self, G_dev, small, want_A, want_v, D):
+    def _run_without(self, G_dev, small, want_A, want_v, D, v0=None):
         """run_device on the spectra above the threshold, results scattered back into full-size tensors."""
         import torch
         B = int(G_dev.shape[0])
@@ -349,8 +364,11 @@ class BatchedTauMaxEnt(object):
             sub.err = np.asarray(self.err)[kept]
         if getattr(self, "cov", None) is not None and self.cov.ndim == 3:
             sub.cov = self.cov[kept]
+        if getattr(self, "_groups", None) is not None:
+            sub.err, sub._groups = self.err, self._groups[kept]
         Dk = None if D is None else (D[keep] if torch.is_tensor(D) else np.asarray(D)[kept])
-        r = sub.run_device(G_dev[keep].contiguous(), want_A=want_A, want_v=want_v, D=Dk) if keep.numel() else None
+        vk = None if v0 is None else v0[keep].contiguous()
+        r = sub.run_device(G_dev[keep].contiguous(), want_A=want_A, want_v=want_v, D=Dk, v0=vk) if keep.numel() else None
         prob = self.prepare()
         dev = prob.device
         n_alpha = len(self.alpha_mesh)

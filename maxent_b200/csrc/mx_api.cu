@@ -229,6 +229,46 @@ __global__ void __launch_bounds__(128) analyze_kernel(const double* __restrict__
     }
 }
 
+// ---- PoormanMaxEnt off-diagonal default models (python/elementwise_maxent.py:633-652), one CTA per spectrum p -------
+// D[p] = (sqrt(A_i A_j) + d_add) * delta from the diagonal pass's analyzer output, and the initial vector
+// v0[p] = V'_g^T log(arg(H0, D[p])) of the plus-minus entropy (engine.per_spectrum_models).  v0 is summed over omega in
+// index order by one thread per singular component, so every spectrum's result is independent of P and of its position.
+__global__ void __launch_bounds__(256) poorman_models_kernel(const double* __restrict__ A_out, int slot,
+                                                             const int32_t* __restrict__ rows,
+                                                             const double* __restrict__ delta, double d_add,
+                                                             const double* __restrict__ A_init,
+                                                             const double* __restrict__ Vp,
+                                                             const int32_t* __restrict__ group, int n_omega, int n_sv,
+                                                             int ldD, double* __restrict__ D, double* __restrict__ v0,
+                                                             int32_t* __restrict__ ok) {
+    extern __shared__ double larg[];    // log(arg) of this spectrum, [n_omega]
+    const int p = blockIdx.x, tid = threadIdx.x;
+    const double* Ai = A_out + ((int64_t)rows[2 * p] * MX_N_ANALYZERS + slot) * n_omega;
+    const double* Aj = A_out + ((int64_t)rows[2 * p + 1] * MX_N_ANALYZERS + slot) * n_omega;
+    double* Dp = D + (int64_t)p * ldD;
+    int nan_seen = 0;
+    for (int w = tid; w < n_omega; w += blockDim.x) {
+        const double ai = Ai[w], aj = Aj[w];
+        nan_seen |= isnan(ai) || isnan(aj);
+        // explicit rounding steps: the same operations, in the same order, as DataDefaultModel(np.sqrt(.) + c).D
+        const double Dw = __dmul_rn(__dadd_rn(__dsqrt_rn(__dmul_rn(ai, aj)), d_add), delta[w]);
+        Dp[w] = Dw;
+        const double H0 = (A_init ? A_init[w] : Dw) * delta[w];      // maxent_loop.py:196-203 quirk
+        double arg = (H0 + sqrt(H0 * H0 + 4.0 * Dw * Dw)) / (2.0 * Dw);   // functions.py:793-796
+        if (fabs(arg) <= 1e-100) arg = 1e-100;
+        larg[w] = log(arg);
+    }
+    for (int w = n_omega + tid; w < ldD; w += blockDim.x) Dp[w] = 0.0;
+    const int any_nan = __syncthreads_or(nan_seen);
+    if (tid == 0) ok[p] = any_nan ? 0 : 1;
+    const double* V = Vp + (group ? (int64_t)group[p] * n_omega * n_sv : 0);
+    for (int k = tid; k < n_sv; k += blockDim.x) {
+        double acc = 0.0;
+        for (int w = 0; w < n_omega; ++w) acc = fma(V[(int64_t)w * n_sv + k], larg[w], acc);
+        v0[(int64_t)p * n_sv + k] = acc;
+    }
+}
+
 // ---- measurement helper: FP64 pipe peak (the roofline denominator of the sweep kernel) --------------------------
 // Every SM runs 2 x 8 warps of independent DMMA (m8n8k4) or DFMA chains: what the FP64 pipe delivers when nothing else
 // limits it.  bench.py calls this inside the benchmark run (MEASURED_PEAKS.json carries no FP64 figure).
@@ -453,6 +493,22 @@ int mx_analyze(const double* alpha, const double* chi2, const double* S, const d
     const size_t shb = 4 * (size_t)n_alpha * sizeof(double);
     analyze_kernel<<<B, 128, shb, (cudaStream_t)stream>>>(alpha, chi2, S, logp, A, n_alpha, n_omega, gamma,
                                                           linefit_deg, bryan_by_integration, alpha_index, A_out, aux);
+    return cudaGetLastError() == cudaSuccess ? MX_OK : MX_ERR_CUDA;
+}
+
+int mx_poorman_models(const double* A_out, int32_t slot, const int32_t* rows, int32_t P, const double* delta,
+                      double d_add, const double* A_init, const double* Vp, const int32_t* group, int32_t n_omega,
+                      int32_t n_sv, double* D, double* v0, int32_t* ok, void* stream) {
+    if (P == 0) return MX_OK;
+    if (!A_out || !rows || !delta || !Vp || !D || !v0 || !ok || P < 0 || slot < 0 || slot >= MX_N_ANALYZERS
+        || n_omega < 1 || n_sv < 1 || n_sv > MX_MAX_NSV) return MX_ERR_BAD_ARG;
+    const size_t shb = (size_t)n_omega * sizeof(double);
+    if (shb > 227 * 1024) return MX_ERR_UNSUPPORTED;
+    if (shb > 48 * 1024 &&
+        cudaFuncSetAttribute(poorman_models_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shb) != cudaSuccess)
+        return MX_ERR_CUDA;
+    poorman_models_kernel<<<P, 256, shb, (cudaStream_t)stream>>>(A_out, slot, rows, delta, d_add, A_init, Vp, group,
+                                                                 n_omega, n_sv, (n_omega + 1) & ~1, D, v0, ok);
     return cudaGetLastError() == cudaSuccess ? MX_OK : MX_ERR_CUDA;
 }
 

@@ -407,6 +407,17 @@ def per_spectrum_models(prob, D, A_init=None):
     return D_rows, v0_rows
 
 
+def _model_rows(D, v0, B, ld, s, dev):
+    """Per-spectrum model rows handed over ready-made: D[B, ldD], v0[B, n_sv] (v0 zero-padded to a padded view's n_sv)."""
+    torch = _torch()
+    if D is None or tuple(D.shape) != (B, ld) or v0.shape[0] != B or v0.shape[1] > s:
+        raise ValueError("ready-made model rows must be D[%d, %d] and v0[%d, <= %d]" % (B, ld, B, s))
+    D, v0 = _dev_f64(D, dev), _dev_f64(v0, dev)
+    if v0.shape[1] < s:
+        v0 = torch.cat([v0, torch.zeros((B, s - v0.shape[1]), dtype=v0.dtype, device=dev)], dim=1).contiguous()
+    return D, v0
+
+
 def project_data(prob, G):
     """mx_project_data: gt[B, n_sv] = (sqrt(W) Q)^T G and c0[B] = the part of chi2 outside the kept
     singular space (NormalChi2.f uses the full kernel, python/functions.py:358-360)."""
@@ -450,7 +461,7 @@ def analyze(alpha, chi2, S, logp, A, gamma=0.2, linefit_deg=0, bryan_by_integrat
 
 def run_sweep(prob, G, alpha_eff, probability=False, lm=None, chi2_factor=1.0, want_A=True, want_v=True,
               analyze_results=True, gamma=0.2, linefit_deg=0, bryan_by_integration=False, time_kernel=False, D=None,
-              phase_timers=False, sigma=None, groups=None, alpha_scale=None):
+              phase_timers=False, sigma=None, groups=None, alpha_scale=None, v0=None):
     """Fused alpha sweep for a batch G[B, n_tau] sharing `prob`.  `alpha_eff` = alpha * scale_alpha, descending.
     G may live on the host (numpy / pinned tensor: copied asynchronously) or on the device.
     Everything stays on the device; returns a SweepResult of torch tensors.
@@ -461,7 +472,11 @@ def run_sweep(prob, G, alpha_eff, probability=False, lm=None, chi2_factor=1.0, w
     or covariance (hence in the whitening rotation V'); G[b] is then the data of spectrum b in the (rotated) data space
     of its group, rows padded to the longest.  ``prob`` must be problems[0].  ``alpha_scale`` [B] (with ``groups``)
     multiplies the alpha mesh per spectrum (scale_alpha = 'Ndata' when groups keep different numbers of data rows; the
-    analyzers are invariant under a common factor on alpha and see the unscaled mesh)."""
+    analyzers are invariant under a common factor on alpha and see the unscaled mesh).
+
+    Default models per spectrum: ``D`` [B, n_omega] (incl. delta omega), with or without ``groups``; every spectrum's
+    initial vector is computed in the basis of its own group's V'.  With ``v0`` [B, n_sv] the rows are already built on
+    the device (``D`` then [B, ldD] in the MX_PER_SPECTRUM_MODEL layout, e.g. by mx_poorman_models)."""
     torch = _torch()
     lib = prob.lib
     dev = prob.device
@@ -490,8 +505,6 @@ def run_sweep(prob, G, alpha_eff, probability=False, lm=None, chi2_factor=1.0, w
             index = torch.as_tensor(np.asarray(index) if not torch.is_tensor(index) else index, device=dev).to(torch.int64)
             if probs[0] is not prob or any(q.n_sv != s or q.n_omega != n_omega or q.variant != prob.variant for q in probs):
                 raise ValueError("the problems of all groups must share the omega mesh and the cost function")
-            if D is not None:
-                raise ValueError("per-spectrum default models and error groups cannot be combined yet")
             nvt = max(int(q.Vt.numel()) for q in probs)
             rows.Vt = torch.zeros((len(probs), nvt), dtype=f64, device=dev)
             for g, q in enumerate(probs):
@@ -500,14 +513,28 @@ def run_sweep(prob, G, alpha_eff, probability=False, lm=None, chi2_factor=1.0, w
             if alpha_scale is not None:          # alpha * (data rows of the spectrum's group), python/maxent_loop.py:216-220
                 rows.alpha = (alpha[None, :] * _dev_f64(alpha_scale, dev).reshape(-1, 1)).contiguous()
             rows.xi = torch.stack([q.xi for q in probs])[index].contiguous()
-            rows.v0 = torch.stack([q.v0 for q in probs])[index].contiguous()
             ld = (n_omega + 1) & ~1
-            rows.D = torch.zeros((B, ld), dtype=f64, device=dev)
-            rows.D[:, :n_omega] = prob.D
+            if v0 is not None:
+                rows.D, rows.v0 = _model_rows(D, v0, B, ld, s, dev)
+            elif D is not None:
+                D = _dev_f64(D, dev)
+                if tuple(D.shape) != (B, n_omega):
+                    raise ValueError("D must be [%d, %d]" % (B, n_omega))
+                rows.D = torch.zeros((B, ld), dtype=f64, device=dev)
+                rows.v0 = torch.zeros((B, s), dtype=f64, device=dev)
+            else:
+                rows.v0 = torch.stack([q.v0 for q in probs])[index].contiguous()
+                rows.D = torch.zeros((B, ld), dtype=f64, device=dev)
+                rows.D[:, :n_omega] = prob.D
             for g, q in enumerate(probs):              # projection per group: its own Q, 1/err and row count
                 sel = torch.nonzero(index == g).flatten()
                 if sel.numel() == 0:
                     continue
+                if D is not None and v0 is None:       # the spectrum's own model, v0 in its group's basis
+                    qb = getattr(q, "base", q)
+                    Dg, vg = per_spectrum_models(qb, D[sel], getattr(qb, "A_init_host", None))
+                    rows.D[sel] = Dg
+                    rows.v0[sel, :qb.n_sv] = vg
                 Gg = G[sel][:, :q.n_tau].contiguous()
                 qq = getattr(q, "base", q)                 # projection in the group's own (unpadded) singular space
                 gg = torch.empty((sel.numel(), qq.n_sv), dtype=f64, device=dev)
@@ -519,7 +546,9 @@ def run_sweep(prob, G, alpha_eff, probability=False, lm=None, chi2_factor=1.0, w
         else:
             if G.shape[1] != prob.n_tau:
                 raise ValueError("G has %d data points, kernel has %d" % (G.shape[1], prob.n_tau))
-            if D is not None:                    # one default model per spectrum, D[B, n_omega]
+            if v0 is not None:                   # rows built on the device already
+                rows.D, rows.v0 = _model_rows(D, v0, B, (n_omega + 1) & ~1, s, dev)
+            elif D is not None:                  # one default model per spectrum, D[B, n_omega]
                 rows.D, rows.v0 = per_spectrum_models(prob, D, getattr(prob, "A_init_host", None))
                 if rows.D.shape[0] != B:
                     raise ValueError("D has %d rows for %d spectra" % (rows.D.shape[0], B))

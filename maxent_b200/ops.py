@@ -3,6 +3,7 @@
     torch.ops.maxent_b200.project_data    -> mx_project_data
     torch.ops.maxent_b200.alpha_sweep     -> mx_alpha_sweep
     torch.ops.maxent_b200.analyze         -> mx_analyze
+    torch.ops.maxent_b200.poorman_models  -> mx_poorman_models
 
 The operators are registered for the CUDA dispatch key ONLY: calling one with host tensors raises
 ``NotImplementedError`` from the dispatcher -- there is no CPU implementation of the hot path.  They are thin:
@@ -33,6 +34,8 @@ _library.define("alpha_sweep(" + _PROBLEM + ", Tensor gt, Tensor c0, Tensor(a!)?
                 "Tensor(n!) workspace) -> ()")
 _library.define("analyze(Tensor alpha, Tensor chi2, Tensor S, Tensor? logp, Tensor? A, float gamma, int linefit_deg, "
                 "bool bryan_by_integration, Tensor(a!) alpha_index, Tensor(b!)? A_out, Tensor(c!)? aux) -> ()")
+_library.define("poorman_models(Tensor A_out, int slot, Tensor rows, Tensor delta, float d_add, Tensor? A_init, Tensor Vp, "
+                "Tensor? group, Tensor(a!) D, Tensor(b!) v0, Tensor(c!) ok) -> ()")
 
 
 def _ptr(t):
@@ -92,11 +95,51 @@ def _analyze(alpha, chi2, S, logp, A, gamma, linefit_deg, bryan_by_integration, 
                                           _ptr(alpha_index), _ptr(A_out), _ptr(aux), _stream(chi2)), "mx_analyze")
 
 
+def _poorman_models(A_out, slot, rows, delta, d_add, A_init, Vp, group, D, v0, ok):
+    """``rows`` [P, 2] and ``group`` [P] are HOST tensors: every index the kernel dereferences is checked here before
+    they are uploaded (rows within the R spectra of A_out[R, 5, n_omega], group within the G buffers of
+    Vp[G, n_omega, n_sv]), so the check needs nothing back from the device."""
+    _f64c(A_out, delta, A_init, Vp, D, v0)
+    for t in (rows, group, ok):
+        if t is not None and (t.dtype != torch.int32 or not t.is_contiguous()):
+            raise ValueError("rows, group and ok must be contiguous int32 tensors")
+    if rows.is_cuda or (group is not None and group.is_cuda):
+        raise ValueError("rows and group must be host tensors (their bounds are checked before the upload)")
+    if A_out.dim() != 3 or A_out.shape[1] != _lib.N_ANALYZERS or not 0 <= int(slot) < _lib.N_ANALYZERS:
+        raise ValueError("A_out must be [R, %d, n_omega] and slot an analyzer index" % _lib.N_ANALYZERS)
+    R, n_omega = int(A_out.shape[0]), int(A_out.shape[2])
+    if Vp.dim() == 2:
+        Vp = Vp[None]
+    G, n_sv = int(Vp.shape[0]), int(Vp.shape[2])
+    P = int(rows.shape[0])
+    ldD = (n_omega + 1) & ~1
+    if rows.shape != (P, 2) or Vp.shape[1] != n_omega or delta.numel() != n_omega:
+        raise ValueError("rows must be [P, 2], Vp [G, n_omega, n_sv] and delta [n_omega]")
+    if A_init is not None and A_init.numel() != n_omega:
+        raise ValueError("A_init must have n_omega points")
+    if D.shape != (P, ldD) or v0.shape != (P, n_sv) or ok.shape != (P,):
+        raise ValueError("D must be [P, %d] (n_omega rounded up to even), v0 [P, n_sv], ok [P]" % ldD)
+    if (group is None and G != 1) or (group is not None and group.shape != (P,)):
+        raise ValueError("group must be [P] (or None with a single V' buffer)")
+    if P == 0:
+        return
+    if int(rows.min()) < 0 or int(rows.max()) >= R or (group is not None and (int(group.min()) < 0 or int(group.max()) >= G)):
+        raise ValueError("rows must lie in [0, %d) and group in [0, %d)" % (R, G))
+    rows = rows.to(A_out.device, non_blocking=True)
+    group = None if group is None else group.to(A_out.device, non_blocking=True)
+    with torch.cuda.device(A_out.device):
+        _lib.check(_lib.load().mx_poorman_models(_ptr(A_out), int(slot), _ptr(rows), P, _ptr(delta), float(d_add),
+                                                 _ptr(A_init), _ptr(Vp), _ptr(group), n_omega, n_sv,
+                                                 _ptr(D), _ptr(v0), _ptr(ok), _stream(A_out)), "mx_poorman_models")
+
+
 _library.impl("project_data", _project_data, "CUDA")
 _library.impl("alpha_sweep", _alpha_sweep, "CUDA")
 _library.impl("analyze", _analyze, "CUDA")
+_library.impl("poorman_models", _poorman_models, "CUDA")
 
 project_data = torch.ops.maxent_b200.project_data
 alpha_sweep = torch.ops.maxent_b200.alpha_sweep
 analyze = torch.ops.maxent_b200.analyze
-OPERATORS = ("project_data", "alpha_sweep", "analyze")
+poorman_models = torch.ops.maxent_b200.poorman_models
+OPERATORS = ("project_data", "alpha_sweep", "analyze", "poorman_models")
