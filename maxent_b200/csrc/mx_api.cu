@@ -85,7 +85,8 @@ __device__ double line_resid(const double* x, const double* y, int i0, int i1, i
     double sxx = 0, sxy = 0, syy = 0;
     for (int i = i0; i < i1; ++i) if (!isnan(y[i])) { const double dx = x[i] - mx, dy = y[i] - my; sxx += dx * dx; sxy += dx * dy; syy += dy * dy; }
     if (deg == 0) { *slope = 0.0; *icpt = my; return n > 1 ? syy : 0.0; }
-    if (n < 2 || sxx == 0.0) { *slope = 0.0; *icpt = my; return 0.0; }
+    // one point (or all x equal): np.polyfit returns the minimum-norm line of its column-scaled problem, y / (2x) and y / 2
+    if (n < 2 || sxx == 0.0) { *slope = mx != 0.0 ? my / (2.0 * mx) : 0.0; *icpt = mx != 0.0 ? 0.5 * my : my; return 0.0; }
     const double m = sxy / sxx;
     *slope = m; *icpt = my - m * mx;
     double r = 0;

@@ -493,6 +493,11 @@ def run_sweep(prob, G, alpha_eff, probability=False, lm=None, chi2_factor=1.0, w
             # groups with different singular-space dimensions (different kernels, e.g. the b values of a preblur scan):
             # every group is padded with zero columns of V' (and zero xi, v0, g~) up to the largest.  The padded
             # components never move (their rows of Z, J and f are exactly zero) and add exact zeros to every sum.
+            # Not for the Bryan cost function (its gradient divides by xi: 0 / 0 in a padded component) nor for
+            # Marquardt's damping mu diag(J) (an exact zero pivot in a padded row): those need one launch per n_sv.
+            if prob.variant == "bryan" or lm.marquardt:
+                raise ValueError("groups of different n_sv cannot share a launch with the Bryan cost function or "
+                                 "Marquardt's damping: run each n_sv separately")
             s = max(q.n_sv for q in groups[0])
             prob = _PaddedView(prob, s)
             groups = ([prob] + [_PaddedView(q, s) for q in groups[0][1:]], groups[1])

@@ -166,7 +166,9 @@ class MaxEntLoop(object):
                 groups.append([job])
         # Consecutive groups that differ only in their device problem (other kernel, other error model: e.g. the b values
         # of a preblur scan, doc/guide/preblur_example.py:46-75) and use the problem's own default model go through ONE
-        # launch of the sweep as whitening groups (engine.run_sweep(groups=...)).
+        # launch of the sweep as whitening groups (engine.run_sweep(groups=...)).  Groups of different n_sv are padded to
+        # the largest, which is not exact for the Bryan cost function nor for Marquardt's damping: there only problems of
+        # the same n_sv share a launch.
         merged = []
         for group in groups:
             p0 = group[0]["problem"]
@@ -175,6 +177,7 @@ class MaxEntLoop(object):
             if (last is not None and last["multi_ok"] and own_D and last["jobs"][0]["scale"] == group[0]["scale"]
                     and last["jobs"][0]["problem"].variant == p0.variant and last["jobs"][0]["problem"].n_omega == p0.n_omega
                     and last["jobs"][0]["problem"].n_tau == p0.n_tau
+                    and (last["jobs"][0]["problem"].n_sv == p0.n_sv or not (p0.variant == "bryan" or lm.marquardt))
                     and np.array_equal(last["jobs"][0]["problem"].D_host, p0.D_host)):
                 last["jobs"].extend(group)
             else:
