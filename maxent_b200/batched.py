@@ -102,6 +102,22 @@ class BatchedMaxEntResult(object):
         return d
 
 
+class _BatchPlan(object):
+    """The error model of one launch: ``problems`` (its SharedProblems; the base problem alone without whitening groups),
+    ``index`` [B] (host: every spectrum's problem) or None, ``sigma`` [B] or None, ``alpha`` (the mesh the sweep gets),
+    ``alpha_scale`` [B] or None, and ``rotations``: per group the rotation T of the data of a covariance group, or None."""
+
+    def __init__(self, problems, index, sigma, alpha, alpha_scale=None, rotations=None):
+        self.problems, self.index, self.sigma = problems, index, sigma
+        self.alpha, self.alpha_scale, self.rotations = alpha, alpha_scale, rotations
+
+    def subset(self, rows):
+        """The plan of the spectra `rows` (host indices): the same problems under the same numbering."""
+        take = lambda x: None if x is None else x[rows]
+        return _BatchPlan(self.problems, take(self.index), take(self.sigma), self.alpha, take(self.alpha_scale),
+                          self.rotations)
+
+
 class BatchedTauMaxEnt(object):
     """MaxEnt continuation of a batch G[B, n_tau] sharing tau grid, omega mesh, error model and alpha mesh.
 
@@ -135,6 +151,10 @@ class BatchedTauMaxEnt(object):
         self.beta = None
         self.K = None                     # explicit kernel matrix (DataKernel) or None -> TauKernel(tau, omega, beta)
         self.err = None
+        self.cov = None
+        self._per_spectrum = None
+        self._groups = None               # set_error_groups: the group of every spectrum
+        self._group_cache = {}            # content of a whitening group -> its SharedProblem
         self.G = None
         self.problem = None
         self.gamma, self.linefit_deg, self.bryan_by_integration = 0.2, 0, False
@@ -202,9 +222,12 @@ class BatchedTauMaxEnt(object):
         self._group_cache = {}
 
     def _error_plan(self, B):
-        """-> ('shared', None) | ('sigma', sigma[B]) | ('groups', index[B], [spec_g]) with spec = (T or None, err vector)."""
+        """The error model of B spectra, worked out on the host: ('shared', None, None) | ('sigma', sigma[B], None) |
+        ('groups', index[B], specs) with one spec = (T or None, error vector) per whitening group.  The groups of
+        err[B, n_tau] are numbered in the sorted order of their vectors, those of cov[B, n, n] in the order of first
+        appearance."""
         n_tau = len(self.tau) if self.tau is not None else self.K.shape[0]
-        if getattr(self, "cov", None) is not None:
+        if self.cov is not None:
             covs = self.cov if self.cov.ndim == 3 else self.cov[None]
             if self.cov.ndim == 3 and covs.shape[0] != B:
                 raise Exception("%d covariance matrices for %d spectra" % (covs.shape[0], B))
@@ -223,7 +246,7 @@ class BatchedTauMaxEnt(object):
         if self.err is None:
             raise Exception("no error set: call set_error")
         err = np.asarray(self.err, dtype=np.float64)
-        if getattr(self, "_groups", None) is not None:
+        if self._groups is not None:
             if self._groups.shape != (B,) or err.ndim != 2 or err.shape[1] != n_tau:
                 raise Exception("error groups: %s vectors for %d spectra, index %s" % (err.shape, B, self._groups.shape))
             return "groups", self._groups, [(None, e) for e in err]
@@ -237,6 +260,27 @@ class BatchedTauMaxEnt(object):
             raise Exception("error array has shape %s, data has %s" % (err.shape, (B, n_tau)))
         uniq, index = np.unique(err, axis=0, return_inverse=True)
         return "groups", np.asarray(index).reshape(-1), [(None, u) for u in uniq]
+
+    def _batch_plan(self, B):
+        """The error model of a launch over B spectra (_error_plan) with the SharedProblem of every group and the
+        alpha mesh; computed on the whole batch, so that a spectrum's group does not depend on which others are live."""
+        mode, a, specs = self._error_plan(B)
+        plan = _BatchPlan([self.prepare()], None, a if mode == "sigma" else None, self.alpha_effective())
+        if mode != "groups":
+            return plan
+        plan.index = index = a
+        plan.problems = [self._group_problem(spec) for spec in specs]
+        if specs[0][0] is not None:
+            plan.rotations = [T for T, _ in specs]
+        rows = [q.n_tau for q in plan.problems]
+        if isinstance(self.scale_alpha, str) and len(set(rows)) > 1:
+            # scale_alpha = 'Ndata' counts the rows of the ROTATED data (python/maxent_loop.py:216-220, after set_cov):
+            # groups whose covariance dropped eigenvalues get their own factor
+            plan.alpha = np.asarray(self.alpha_mesh, dtype=np.float64)
+            plan.alpha_scale = np.array([rows[g] for g in index], dtype=np.float64)
+        elif isinstance(self.scale_alpha, str):
+            plan.alpha = np.asarray(self.alpha_mesh, dtype=np.float64) * rows[0]
+        return plan
 
     # ---- run --------------------------------------------------------------------------------------
     def prepare(self):
@@ -266,11 +310,11 @@ class BatchedTauMaxEnt(object):
                                              K.data_ptr(), stream), "mx_tau_kernel")
             else:
                 K = torch.as_tensor(self.K, device=dev)
-        if self.err is None and getattr(self, "cov", None) is None:
+        if self.err is None and self.cov is None:
             raise Exception("no error set: call set_error")
         D = FlatDefaultModel(omega).D if self.D is None else (self.D.D if hasattr(self.D, "D") else np.asarray(self.D))
         err = np.asarray(1.0 if self.err is None else self.err, dtype=np.float64)
-        shared = err.ndim == 0 or (err.ndim == 1 and err.shape[0] == K.shape[0] and not getattr(self, "_per_spectrum", None))
+        shared = err.ndim == 0 or (err.ndim == 1 and err.shape[0] == K.shape[0] and not self._per_spectrum)
         # per-spectrum error models: the base problem carries err = 1 (kernel SVD, truncation, V layout); error scales
         # or whitening groups are attached per launch (run_device)
         self._K_dev, self._D_host = K, D
@@ -279,21 +323,22 @@ class BatchedTauMaxEnt(object):
                                             device=dev, svd=self.svd, A_init=self.A_init)
         return self.problem
 
-    def _group_problem(self, g, spec):
-        """SharedProblem of one whitening group: the base kernel SVD with the group's error vector / covariance rotation."""
+    def _group_problem(self, spec):
+        """SharedProblem of one whitening group: the base kernel SVD with the group's error vector / covariance rotation,
+        cached under the group's content."""
         import torch
-        cache = self.__dict__.setdefault("_group_cache", {})
-        if g in cache:
-            return cache[g]
-        base = self.prepare()
         T, err = spec
-        K, U = self._K_dev, base.U
-        if T is not None:
-            Td = torch.as_tensor(T, device=base.device)
-            K, U = Td @ K, Td @ U
-        cache[g] = engine.SharedProblem(K, err, self._D_host, self.omega.delta, variant=self.cost_function, device=base.device,
-                                        svd=self.svd, A_init=self.A_init, usv=(U, base.S, base.V), orthonormal_U=T is None)
-        return cache[g]
+        key = (None if T is None else T.tobytes(), err.tobytes())
+        if key not in self._group_cache:
+            base = self.prepare()
+            K, U = self._K_dev, base.U
+            if T is not None:
+                Td = torch.as_tensor(T, device=base.device)
+                K, U = Td @ K, Td @ U
+            self._group_cache[key] = engine.SharedProblem(
+                K, err, self._D_host, self.omega.delta, variant=self.cost_function, device=base.device, svd=self.svd,
+                A_init=self.A_init, usv=(U, base.S, base.V), orthonormal_U=T is None)
+        return self._group_cache[key]
 
     def alpha_effective(self):
         """alpha * scale_alpha (python/maxent_loop.py:216-232)."""
@@ -314,68 +359,47 @@ class BatchedTauMaxEnt(object):
         ``skip_small``: spectra with max|G| < G_threshold are NOT continued (python/maxent_loop.py:174-179): they are left
         out of the launch and come back with status MX_STATUS_SKIPPED, NaN scalars, alpha_index -1 and A = 0."""
         import torch
-        if skip_small and G_dev.dim() > 1 and G_dev.shape[0]:
-            small = G_dev.abs().amax(dim=1) < self.G_threshold
+        skip = skip_small and G_dev.dim() > 1
+        G = G_dev if G_dev.dim() > 1 else G_dev[None, :]
+        B = int(G.shape[0])
+        plan = self._batch_plan(B)
+        if skip and B:
+            small = G.abs().amax(dim=1) < self.G_threshold
             if bool(small.any()):
-                return self._run_without(G_dev, small, want_A, want_v, D, v0)
-        prob = self.prepare()
-        kw = dict(probability=self.probability is not None, lm=self.minimizer, want_A=want_A, want_v=want_v,
-                  gamma=self.gamma, linefit_deg=self.linefit_deg, bryan_by_integration=self.bryan_by_integration, D=D,
-                  v0=v0)
-        B = int(G_dev.shape[0]) if G_dev.dim() > 1 else 1
-        mode, a, specs = self._error_plan(B)
-        if mode == "shared":
-            return engine.run_sweep(prob, G_dev, self.alpha_effective(), **kw)
-        if mode == "sigma":
-            return engine.run_sweep(prob, G_dev, self.alpha_effective(), sigma=a, **kw)
-        probs = [self._group_problem(g, spec) for g, spec in enumerate(specs)]
-        Gd = G_dev if G_dev.dim() > 1 else G_dev[None, :]
-        if any(spec[0] is not None for spec in specs):        # covariance groups: rotate the data, G' = T_g G
-            rows = max(q.n_tau for q in probs)
-            Gr = torch.zeros((B, rows), dtype=torch.float64, device=Gd.device)
-            idx = torch.as_tensor(a, device=Gd.device)
-            for g, (T, _) in enumerate(specs):
-                sel = torch.nonzero(idx == g).flatten()
-                if sel.numel():
-                    Gr[sel, :probs[g].n_tau] = Gd[sel] @ torch.as_tensor(T, device=Gd.device).T
-            Gd = Gr
-        alpha, scale = self.alpha_effective(), None
-        if isinstance(self.scale_alpha, str) and len(set(q.n_tau for q in probs)) > 1:
-            # scale_alpha = 'Ndata' counts the rows of the ROTATED data (python/maxent_loop.py:216-220, after set_cov):
-            # groups whose covariance dropped eigenvalues get their own factor
-            alpha = np.asarray(self.alpha_mesh, dtype=np.float64)
-            scale = np.array([probs[g].n_tau for g in a], dtype=np.float64)
-        elif isinstance(self.scale_alpha, str):
-            alpha = np.asarray(self.alpha_mesh, dtype=np.float64) * probs[0].n_tau
-        res = engine.run_sweep(probs[0], Gd, alpha, groups=(probs, a), alpha_scale=scale, **kw)
-        res.alpha_scale = scale
-        return res
+                keep = torch.nonzero(~small).flatten()
+                kept = keep.cpu().numpy()
+                Dk = None if D is None else (D[keep] if torch.is_tensor(D) else np.asarray(D)[kept])
+                vk = None if v0 is None else v0[keep].contiguous()
+                r = self._launch(plan.subset(kept), G[keep].contiguous(), want_A, want_v, Dk, vk) if len(kept) else None
+                return self._scatter(r, keep, plan, B, want_A, want_v)
+        return self._launch(plan, G, want_A, want_v, D, v0)
 
-    def _run_without(self, G_dev, small, want_A, want_v, D, v0=None):
-        """run_device on the spectra above the threshold, results scattered back into full-size tensors."""
+    def _launch(self, plan, G, want_A, want_v, D, v0):
         import torch
-        B = int(G_dev.shape[0])
-        keep = torch.nonzero(~small).flatten()
-        kept = keep.cpu().numpy()
-        sub = BatchedTauMaxEnt.__new__(BatchedTauMaxEnt)
-        sub.__dict__.update(self.__dict__)                     # same kernel / problem caches, error model rows subset
-        if self.err is not None and np.ndim(self.err) >= 1 and np.shape(self.err)[0] == B and \
-                (np.ndim(self.err) == 2 or self._per_spectrum or B != self.prepare().n_tau):
-            sub.err = np.asarray(self.err)[kept]
-        if getattr(self, "cov", None) is not None and self.cov.ndim == 3:
-            sub.cov = self.cov[kept]
-        if getattr(self, "_groups", None) is not None:
-            sub.err, sub._groups = self.err, self._groups[kept]
-        Dk = None if D is None else (D[keep] if torch.is_tensor(D) else np.asarray(D)[kept])
-        vk = None if v0 is None else v0[keep].contiguous()
-        r = sub.run_device(G_dev[keep].contiguous(), want_A=want_A, want_v=want_v, D=Dk, v0=vk) if keep.numel() else None
+        if plan.rotations is not None:           # covariance groups: rotate the data, G' = T_g G
+            Gr = torch.zeros((G.shape[0], max(q.n_tau for q in plan.problems)), dtype=torch.float64, device=G.device)
+            for g, T in enumerate(plan.rotations):
+                sel = torch.as_tensor(np.nonzero(plan.index == g)[0], device=G.device)
+                if len(sel):
+                    Gr[sel, :plan.problems[g].n_tau] = G[sel] @ torch.as_tensor(T, device=G.device).T
+            G = Gr
+        return engine.run_sweep(plan.problems[0], G, plan.alpha, probability=self.probability is not None,
+                                lm=self.minimizer, want_A=want_A, want_v=want_v, gamma=self.gamma,
+                                linefit_deg=self.linefit_deg, bryan_by_integration=self.bryan_by_integration, D=D, v0=v0,
+                                sigma=plan.sigma, groups=None if plan.index is None else (plan.problems, plan.index),
+                                alpha_scale=plan.alpha_scale)
+
+    def _scatter(self, r, keep, plan, B, want_A, want_v):
+        """The result `r` of the spectra `keep` of a batch of B, in full-size tensors; the other spectra come back
+        skipped."""
+        import torch
         prob = self.prepare()
         dev = prob.device
         n_alpha = len(self.alpha_mesh)
         full = engine.SweepResult()
         full.alpha = torch.as_tensor(self.alpha_effective(), device=dev) if r is None else r.alpha
         full.n_sv = prob.n_sv
-        full.alpha_scale = None
+        full.alpha_scale, full.problems, full.index = plan.alpha_scale, plan.problems, plan.index
 
         def blank(shape, dtype, fill):
             return torch.full((B,) + shape, fill, dtype=dtype, device=dev)

@@ -133,7 +133,7 @@ class BatchedMatrixMaxEntResult(object):
             if res is None or self._not_run[k][r]:
                 continue
             worker = self._workers[k]
-            prob = self._row_problem[k](r)
+            prob = res.problem(r)
             A = res.A[r]
             Kd = worker._K_dev * prob.delta[None, :]
             v = None if res.v is None else prob.v_to_reference_basis(res.v[r][..., :prob.n_sv]).cpu().numpy()
@@ -353,21 +353,8 @@ class BatchedElementwiseMaxEnt(object):
             host.append(got)
         out._not_run = not_run
         out._G_rows = [None if g is None else g.cpu().numpy() for g in G_rows]
-        out._row_problem = [None if res is None else self._row_problem(w, len(plan))
-                            for w, plan, res in zip(self._workers(), plans, results)]
         self._fill(out, plans, host, B, M)
         return out
-
-    @staticmethod
-    def _row_problem(worker, n_rows):
-        """row -> the SharedProblem its sweep ran with (its whitening group's, if any)."""
-        base = worker.prepare()
-        if n_rows == 0 or worker.err is None and getattr(worker, "cov", None) is None:
-            return lambda r: base
-        mode, index, specs = worker._error_plan(n_rows)
-        if mode != "groups":
-            return lambda r: base
-        return lambda r: worker._group_problem(int(index[r]), specs[int(index[r])])
 
     def _fill(self, out, plans, host, B, M):
         n_alpha, n_omega = len(out.alpha), len(self.omega)
@@ -448,12 +435,9 @@ class BatchedPoormanMaxEnt(BatchedElementwiseMaxEnt):
         # indices the kernel dereferences stay on the host: the operator checks them there before the upload
         rows = torch.from_numpy(np.stack([off_plan[:, 0] * M + off_plan[:, 1], off_plan[:, 0] * M + off_plan[:, 2]],
                                          axis=1).astype(np.int32))
-        mode, index, specs = off._error_plan(P)
-        if mode == "groups":
-            Vp = torch.stack([off._group_problem(g, s).Vp for g, s in enumerate(specs)]).contiguous()
-            group = torch.from_numpy(np.asarray(index).astype(np.int32))
-        else:
-            Vp, group = prob.Vp[None].contiguous(), None
+        plan = off._batch_plan(P)
+        Vp = torch.stack([q.Vp for q in plan.problems]).contiguous()
+        group = None if plan.index is None else torch.from_numpy(np.asarray(plan.index).astype(np.int32))
         A_init = None if off.A_init is None else torch.as_tensor(np.asarray(off.A_init, dtype=np.float64), device=dev)
         ld = (prob.n_omega + 1) & ~1
         D = torch.empty((P, ld), dtype=torch.float64, device=dev)

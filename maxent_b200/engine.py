@@ -141,22 +141,9 @@ class SharedProblem(object):
             self.xi = Xi.contiguous()
             self.D = torch.as_tensor(np.asarray(D, dtype=np.float64), dtype=f64, device=dev).contiguous()
             self.delta = torch.as_tensor(np.asarray(delta, dtype=np.float64), dtype=f64, device=dev).contiguous()
-            # ---- initial v (python/maxent_loop.py:196-203; quirk: D*delta although D holds delta) ----
-            self.A_init_host = None if A_init is None else np.asarray(A_init, dtype=np.float64)
-            H0 = (self.D if A_init is None else torch.as_tensor(np.asarray(A_init, dtype=np.float64), device=dev)) * self.delta
-            if variant == "plusminus":
-                arg = (H0 + torch.sqrt(H0**2 + 4 * self.D**2)) / (2 * self.D)   # functions.py:793-796
-            else:
-                arg = H0 / self.D                                               # functions.py:753-755
-            arg = torch.where(arg.abs() <= 1e-100, torch.full_like(arg, 1e-100), arg)
-            self.v0 = (self.Vp.transpose(0, 1) @ torch.log(arg)).contiguous()
-            # ---- re-tile V' for the sweep kernel ----
-            n = int(self.lib.mx_layout_V_size(self.n_omega, s))
-            if n < 0:
-                raise _lib.MaxEntLibraryError("n_sv=%d outside the fused path (max %d)" % (s, _lib.MX_MAX_NSV))
-            self.Vt = torch.empty(n, dtype=f64, device=dev)
-            stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
-            _lib.check(self.lib.mx_layout_V(_ptr(self.Vp), self.n_omega, s, _ptr(self.Vt), stream), "mx_layout_V")
+            self.A_init = None if A_init is None else _dev_f64(A_init, dev)
+            self.v0 = (self.Vp.transpose(0, 1) @ _log_initial_arg(self.D, self.A_init, self.delta, variant)).contiguous()
+            self.Vt = _layout_V(self.lib, self.Vp)
             self.engine = int(engine)
             self.config = _lib.sweep_config(s, self.engine)
 
@@ -187,6 +174,30 @@ class SharedProblem(object):
     def v_to_reference_basis(self, v):
         """v' (rotated basis) -> v in the basis of the truncated SVD of K."""
         return v if self.P is None else v @ self.P.transpose(0, 1)
+
+
+def _log_initial_arg(D, A_init, delta, variant):
+    """log of the argument of the entropy's inverse at the initial H0 = (A_init or D) * delta, with D [..., n_omega]
+    (python/maxent_loop.py:196-203; quirk: D*delta although D holds delta).  The initial vector is V'^T of it."""
+    torch = _torch()
+    H0 = (D if A_init is None else A_init) * delta
+    if variant == "plusminus":
+        arg = (H0 + torch.sqrt(H0 ** 2 + 4 * D ** 2)) / (2 * D)         # functions.py:793-796
+    else:
+        arg = H0 / D                                                     # functions.py:753-755
+    return torch.log(torch.where(arg.abs() <= 1e-100, torch.full_like(arg, 1e-100), arg))
+
+
+def _layout_V(lib, Vp):
+    """V'[n_omega, n_sv] re-tiled for the sweep kernel (mx_layout_V)."""
+    torch = _torch()
+    n_omega, s = int(Vp.shape[0]), int(Vp.shape[1])
+    n = int(lib.mx_layout_V_size(n_omega, s))
+    if n < 0:
+        raise _lib.MaxEntLibraryError("n_sv=%d outside the fused path (max %d)" % (s, _lib.MX_MAX_NSV))
+    Vt = torch.empty(n, dtype=torch.float64, device=Vp.device)
+    _lib.check(lib.mx_layout_V(_ptr(Vp), n_omega, s, _ptr(Vt), _stream(Vp.device)), "mx_layout_V")
+    return Vt
 
 
 def _require_cuda():
@@ -291,39 +302,14 @@ def svd_jacobi_host(K, device=None):
         return U.cpu().numpy(), S.cpu().numpy(), V.cpu().numpy()
 
 
-class _PaddedView(object):
-    """A SharedProblem seen with a larger singular-space dimension: V' re-tiled with zero columns appended, xi and v0
-    zero-padded (see run_sweep, groups of different n_sv).  Everything else is the base problem's."""
-
-    def __init__(self, base, n_sv):
-        torch = _torch()
-        self.base = base
-        self.n_sv = int(n_sv)
-        pad = self.n_sv - base.n_sv
-        dev = base.device
-        z = lambda *shape: torch.zeros(shape, dtype=torch.float64, device=dev)
-        with torch.cuda.device(dev):
-            Vp = torch.cat([base.Vp, z(base.n_omega, pad)], dim=1).contiguous()
-            n = int(base.lib.mx_layout_V_size(base.n_omega, self.n_sv))
-            if n < 0:
-                raise _lib.MaxEntLibraryError("n_sv=%d outside the fused path (max %d)" % (self.n_sv, _lib.MX_MAX_NSV))
-            self.Vt = torch.empty(n, dtype=torch.float64, device=dev)
-            _lib.check(base.lib.mx_layout_V(_ptr(Vp), base.n_omega, self.n_sv, _ptr(self.Vt), _stream(dev)), "mx_layout_V")
-            self.xi = torch.cat([base.xi, z(pad)]).contiguous()
-            self.v0 = torch.cat([base.v0, z(pad)]).contiguous()
-            self.Vp = Vp
-
-    def __getattr__(self, name):                    # n_tau, n_omega, variant, D, delta, Qw, Q, sqrtw, lib, device, ...
-        return getattr(self.base, name)
-
-    def v_to_reference_basis(self, v):
-        return self.base.v_to_reference_basis(v[..., :self.base.n_sv])
-
-
 class SweepResult(object):
-    """Device tensors produced by one call of the fused sweep (+ analyzers)."""
+    """Device tensors produced by one call of the fused sweep (+ analyzers).  ``problems`` and ``index`` (host [B], None
+    for a launch of one problem) say which SharedProblem every spectrum ran with: ``problem(b)``."""
     __slots__ = ("alpha", "v", "A", "chi2", "S", "Q", "logp", "n_iter", "n_qeval", "n_solve", "status",
-                 "alpha_index", "A_out", "n_sv", "n_trial", "n_batch", "phase_cycles", "alpha_scale")
+                 "alpha_index", "A_out", "n_sv", "n_trial", "n_batch", "phase_cycles", "alpha_scale", "problems", "index")
+
+    def problem(self, b):
+        return self.problems[0 if self.index is None else int(self.index[b])]
 
 
 def _stream(dev):
@@ -339,83 +325,26 @@ def _dev_f64(x, dev):
     return torch.as_tensor(np.ascontiguousarray(x, dtype=np.float64), device=dev)
 
 
-class _Rows(object):
-    """Per-spectrum overrides of the shared problem state (MxProblem.per_spectrum_model bits): default models and
-    initial vectors, error scales (xi rows), whitening groups (stacked V' buffers + index)."""
-    __slots__ = ("D", "v0", "xi", "Vt", "vt_index", "vt_stride", "alpha")
-
-    def __init__(self, D=None, v0=None, xi=None, Vt=None, vt_index=None, vt_stride=0, alpha=None):
-        self.D, self.v0, self.xi, self.Vt, self.vt_index, self.vt_stride = D, v0, xi, Vt, vt_index, vt_stride
-        self.alpha = alpha
-
-    def flags(self):
-        return ((_lib.PER_SPECTRUM_MODEL if self.D is not None else 0) | (_lib.PER_SPECTRUM_XI if self.xi is not None else 0)
-                | (_lib.PER_SPECTRUM_VT if self.vt_index is not None else 0)
-                | (_lib.PER_SPECTRUM_ALPHA if self.alpha is not None else 0))
-
-
-def _problem_struct(prob, alpha, probability, lm, chi2_factor, rows=None):
-    r = rows or _Rows()
-    per = r.D is not None
-    return _lib.MxProblem(prob.n_tau, prob.n_omega, prob.n_sv, int(alpha.numel()), _lib.VARIANTS[prob.variant],
-                          int(bool(probability)), int(getattr(prob, "engine", 0)), r.flags(), float(chi2_factor),
-                          _ptr(prob.Vt if r.Vt is None else r.Vt), _ptr(prob.Qw), _ptr(prob.Q), _ptr(prob.sqrtw),
-                          _ptr(prob.xi if r.xi is None else r.xi), _ptr(r.D if per else prob.D), _ptr(prob.delta),
-                          _ptr(alpha if r.alpha is None else r.alpha),
-                          _ptr(r.v0 if per else prob.v0), lm.c_struct(), _ptr(r.vt_index), int(r.vt_stride))
-
-
-def _problem_args(prob, alpha, probability, lm, chi2_factor, rows=None):
-    """The same problem description as the leading arguments of the torch operators (maxent_b200/ops.py)."""
-    r = rows or _Rows()
-    per = r.D is not None
-    dims = [prob.n_tau, prob.n_omega, prob.n_sv, int(alpha.numel()), _lib.VARIANTS[prob.variant],
-            int(bool(probability)), int(getattr(prob, "engine", 0)), r.flags(), int(lm.maxiter), int(lm.miniter),
-            int(lm.marquardt), int(r.vt_stride)]
+def _problem_args(prob, alpha, lm, chi2_factor, probability=False, n_sv=None, Vt=None, xi=None, D=None, v0=None,
+                  vt_index=None, vt_stride=0, alpha_rows=None):
+    """The problem description as the leading arguments of the torch operators (maxent_b200/ops.py): the state of
+    ``prob``, in a singular space of ``n_sv`` dimensions, with the per-spectrum rows that are given in place of its own
+    (MxProblem.per_spectrum_model bits: D with v0, xi, Vt with vt_index, alpha)."""
+    flags = ((_lib.PER_SPECTRUM_MODEL if D is not None else 0) | (_lib.PER_SPECTRUM_XI if xi is not None else 0)
+             | (_lib.PER_SPECTRUM_VT if vt_index is not None else 0)
+             | (_lib.PER_SPECTRUM_ALPHA if alpha_rows is not None else 0))
+    dims = [prob.n_tau, prob.n_omega, prob.n_sv if n_sv is None else n_sv, int(alpha.numel()), _lib.VARIANTS[prob.variant],
+            int(bool(probability)), prob.engine, flags, int(lm.maxiter), int(lm.miniter), int(lm.marquardt), int(vt_stride)]
     params = [float(chi2_factor), float(lm.mu0), float(lm.nu), float(lm.max_mu), float(lm.conv_max_derivative),
               float(lm.conv_rel_change), float(lm.conv_abs_change)]
-    return (prob.Vt if r.Vt is None else r.Vt, prob.Qw, prob.Q, prob.sqrtw, prob.xi if r.xi is None else r.xi,
-            r.D if per else prob.D, prob.delta, alpha if r.alpha is None else r.alpha, r.v0 if per else prob.v0, r.vt_index,
-            dims, params)
+    return (prob.Vt if Vt is None else Vt, prob.Qw, prob.Q, prob.sqrtw, prob.xi if xi is None else xi,
+            prob.D if D is None else D, prob.delta, alpha if alpha_rows is None else alpha_rows,
+            prob.v0 if D is None else v0, vt_index, dims, params)
 
 
 def _ops():
     from . import ops
     return ops
-
-
-def per_spectrum_models(prob, D, A_init=None):
-    """Device buffers for one default model PER SPECTRUM (MxProblem.per_spectrum_model = 1): D[B, n_omega] (incl.
-    delta omega, like DefaultModel.D) -> (D_rows[B, ldD], v0_rows[B, n_sv]); v0 = V'^T log(H0 / D) with
-    H0 = (D or A_init) * delta as in python/maxent_loop.py:196-203 (functions.py:753-755 / 793-796)."""
-    torch = _torch()
-    dev = prob.device
-    D = _dev_f64(D, dev)
-    B, n_omega = int(D.shape[0]), prob.n_omega
-    if D.shape[1] != n_omega:
-        raise ValueError("D has %d points, omega mesh has %d" % (D.shape[1], n_omega))
-    ld = (n_omega + 1) & ~1
-    D_rows = torch.zeros((B, ld), dtype=torch.float64, device=dev)
-    D_rows[:, :n_omega] = D
-    H0 = (D if A_init is None else _dev_f64(A_init, dev)) * prob.delta
-    if prob.variant == "plusminus":
-        arg = (H0 + torch.sqrt(H0 ** 2 + 4 * D ** 2)) / (2 * D)
-    else:
-        arg = H0 / D
-    arg = torch.where(arg.abs() <= 1e-100, torch.full_like(arg, 1e-100), arg)
-    v0_rows = (torch.log(arg) @ prob.Vp).contiguous()
-    return D_rows, v0_rows
-
-
-def _model_rows(D, v0, B, ld, s, dev):
-    """Per-spectrum model rows handed over ready-made: D[B, ldD], v0[B, n_sv] (v0 zero-padded to a padded view's n_sv)."""
-    torch = _torch()
-    if D is None or tuple(D.shape) != (B, ld) or v0.shape[0] != B or v0.shape[1] > s:
-        raise ValueError("ready-made model rows must be D[%d, %d] and v0[%d, <= %d]" % (B, ld, B, s))
-    D, v0 = _dev_f64(D, dev), _dev_f64(v0, dev)
-    if v0.shape[1] < s:
-        v0 = torch.cat([v0, torch.zeros((B, s - v0.shape[1]), dtype=v0.dtype, device=dev)], dim=1).contiguous()
-    return D, v0
 
 
 def project_data(prob, G):
@@ -429,7 +358,7 @@ def project_data(prob, G):
         alpha = torch.ones((1,), dtype=torch.float64, device=dev)
         gt = torch.empty((B, prob.n_sv), dtype=torch.float64, device=dev)
         c0 = torch.empty((B,), dtype=torch.float64, device=dev)
-        _ops().project_data(*_problem_args(prob, alpha, False, LMParams(), 1.0), G, gt, c0)
+        _ops().project_data(*_problem_args(prob, alpha, LMParams(), 1.0), G, gt, c0)
     return gt, c0
 
 
@@ -459,6 +388,8 @@ def analyze(alpha, chi2, S, logp, A, gamma=0.2, linefit_deg=0, bryan_by_integrat
     return idx, A_out
 
 
+
+
 def run_sweep(prob, G, alpha_eff, probability=False, lm=None, chi2_factor=1.0, want_A=True, want_v=True,
               analyze_results=True, gamma=0.2, linefit_deg=0, bryan_by_integration=False, time_kernel=False, D=None,
               phase_timers=False, sigma=None, groups=None, alpha_scale=None, v0=None):
@@ -470,105 +401,115 @@ def run_sweep(prob, G, alpha_eff, probability=False, lm=None, chi2_factor=1.0, w
     launch of the sweep: ``sigma`` [B] gives every spectrum its own scalar error bar (``prob`` built with err = 1);
     ``groups`` = (problems, index[B]) gives every spectrum one of several SharedProblems that differ in the error vector
     or covariance (hence in the whitening rotation V'); G[b] is then the data of spectrum b in the (rotated) data space
-    of its group, rows padded to the longest.  ``prob`` must be problems[0].  ``alpha_scale`` [B] (with ``groups``)
-    multiplies the alpha mesh per spectrum (scale_alpha = 'Ndata' when groups keep different numbers of data rows; the
-    analyzers are invariant under a common factor on alpha and see the unscaled mesh).
+    of its group, rows padded to the longest.  ``prob`` must be problems[0].  ``sigma`` and ``groups`` exclude each
+    other.  ``alpha_scale`` [B] (with ``groups``) multiplies the alpha mesh per spectrum (scale_alpha = 'Ndata' when
+    groups keep different numbers of data rows; the analyzers are invariant under a common factor on alpha and see the
+    unscaled mesh).
 
     Default models per spectrum: ``D`` [B, n_omega] (incl. delta omega), with or without ``groups``; every spectrum's
     initial vector is computed in the basis of its own group's V'.  With ``v0`` [B, n_sv] the rows are already built on
     the device (``D`` then [B, ldD] in the MX_PER_SPECTRUM_MODEL layout, e.g. by mx_poorman_models)."""
     torch = _torch()
-    lib = prob.lib
     dev = prob.device
     f64, i32 = torch.float64, torch.int32
     lm = LMParams() if lm is None else lm
+    ops = _ops()
+    probs, index = ([prob], None) if groups is None else groups
+    if index is not None:
+        if sigma is not None:
+            raise ValueError("sigma and groups cannot be combined: every group carries its own error vector")
+        index = np.asarray(index.cpu() if torch.is_tensor(index) else index)
+    n_omega, s = prob.n_omega, max(q.n_sv for q in probs)
+    if probs[0] is not prob or any(q.n_omega != n_omega or q.variant != prob.variant for q in probs):
+        raise ValueError("the problems of all groups must share the omega mesh and the cost function")
+    if any(q.n_sv != s for q in probs) and (prob.variant == "bryan" or lm.marquardt):
+        # Groups with different singular-space dimensions (different kernels, e.g. the b values of a preblur scan) are
+        # padded with zero columns of V' (and zero xi, v0, g~) up to the largest.  The padded components never move
+        # (their rows of Z, J and f are exactly zero) and add exact zeros to every sum.  Not for the Bryan cost function
+        # (its gradient divides by xi: 0 / 0 in a padded component) nor for Marquardt's damping mu diag(J) (an exact
+        # zero pivot in a padded row): those need one launch per n_sv.
+        raise ValueError("groups of different n_sv cannot share a launch with the Bryan cost function or "
+                         "Marquardt's damping: run each n_sv separately")
     with torch.cuda.device(dev):
         G = _dev_f64(G, dev)
         if G.dim() == 1:
             G = G[None, :]
         B = int(G.shape[0])
         alpha = _dev_f64(np.asarray(alpha_eff, dtype=np.float64) if not torch.is_tensor(alpha_eff) else alpha_eff, dev)
-        n_alpha, s, n_omega = int(alpha.numel()), prob.n_sv, prob.n_omega
-        if groups is not None and any(q.n_sv != s for q in groups[0]):
-            # groups with different singular-space dimensions (different kernels, e.g. the b values of a preblur scan):
-            # every group is padded with zero columns of V' (and zero xi, v0, g~) up to the largest.  The padded
-            # components never move (their rows of Z, J and f are exactly zero) and add exact zeros to every sum.
-            # Not for the Bryan cost function (its gradient divides by xi: 0 / 0 in a padded component) nor for
-            # Marquardt's damping mu diag(J) (an exact zero pivot in a padded row): those need one launch per n_sv.
-            if prob.variant == "bryan" or lm.marquardt:
-                raise ValueError("groups of different n_sv cannot share a launch with the Bryan cost function or "
-                                 "Marquardt's damping: run each n_sv separately")
-            s = max(q.n_sv for q in groups[0])
-            prob = _PaddedView(prob, s)
-            groups = ([prob] + [_PaddedView(q, s) for q in groups[0][1:]], groups[1])
-        rows = _Rows()
-        ops = _ops()
-        gt = torch.empty((B, s), dtype=f64, device=dev)
-        c0 = torch.empty((B,), dtype=f64, device=dev)
-        if groups is not None:
-            probs, index = groups
-            index = torch.as_tensor(np.asarray(index) if not torch.is_tensor(index) else index, device=dev).to(torch.int64)
-            if probs[0] is not prob or any(q.n_sv != s or q.n_omega != n_omega or q.variant != prob.variant for q in probs):
-                raise ValueError("the problems of all groups must share the omega mesh and the cost function")
-            nvt = max(int(q.Vt.numel()) for q in probs)
-            rows.Vt = torch.zeros((len(probs), nvt), dtype=f64, device=dev)
+        n_alpha = int(alpha.numel())
+        zeros = lambda *shape: torch.zeros(shape, dtype=f64, device=dev)
+        # the spectra of every problem: the whole batch for a single problem, the rows of its group otherwise
+        if index is None:
+            if G.shape[1] != prob.n_tau:
+                raise ValueError("G has %d data points, kernel has %d" % (G.shape[1], prob.n_tau))
+            parts = [(prob, slice(None))]
+        else:
+            index_d = torch.as_tensor(index, device=dev).to(torch.int64)
+            parts = []
             for g, q in enumerate(probs):
-                rows.Vt[g, :q.Vt.numel()] = q.Vt
-            rows.vt_index, rows.vt_stride = index.to(torch.int32).contiguous(), nvt
+                sel = np.nonzero(index == g)[0]
+                if len(sel):
+                    parts.append((q, torch.as_tensor(sel, device=dev)))
+        if sigma is not None:                    # Xi_b = Xi / sigma_b, data divided by sigma_b (prob carries err = 1)
+            sg = _dev_f64(sigma, dev).reshape(-1)
+            if sg.numel() != B:
+                raise ValueError("sigma has %d entries for %d spectra" % (sg.numel(), B))
+            G = (G / sg[:, None]).contiguous()
+        # ---- projection: every problem with its own Q, 1/err and data rows, in its own singular space ----
+        gt = torch.empty((B, s), dtype=f64, device=dev) if index is None else zeros(B, s)
+        c0 = torch.empty((B,), dtype=f64, device=dev)
+        for q, sel in parts:
+            if index is None:
+                Gq, gq, cq = G, gt, c0
+            else:
+                Gq = G[sel][:, :q.n_tau].contiguous()
+                gq, cq = torch.empty((len(sel), q.n_sv), dtype=f64, device=dev), torch.empty((len(sel),), dtype=f64, device=dev)
+            ops.project_data(*_problem_args(q, alpha, lm, chi2_factor), Gq, gq, cq)
+            if index is not None:
+                gt[sel, :q.n_sv], c0[sel] = gq, cq
+        # ---- per-spectrum rows, zero-padded to the common n_sv ----
+        xi = Vt = vt_index = alpha_rows = None
+        vt_stride = 0
+        if sigma is not None:
+            xi = (prob.xi[None, :] / sg[:, None]).contiguous()
+        if index is not None:
+            xi = zeros(B, s)
+            for q, sel in parts:
+                xi[sel, :q.n_sv] = q.xi
+            tiled = [q.Vt if q.n_sv == s else _layout_V(q.lib, torch.cat([q.Vp, zeros(n_omega, s - q.n_sv)], dim=1))
+                     for q in probs]
+            vt_stride = max(int(t.numel()) for t in tiled)
+            Vt = zeros(len(probs), vt_stride)
+            for g, t in enumerate(tiled):
+                Vt[g, :t.numel()] = t
+            vt_index = index_d.to(i32).contiguous()
             if alpha_scale is not None:          # alpha * (data rows of the spectrum's group), python/maxent_loop.py:216-220
-                rows.alpha = (alpha[None, :] * _dev_f64(alpha_scale, dev).reshape(-1, 1)).contiguous()
-            rows.xi = torch.stack([q.xi for q in probs])[index].contiguous()
-            ld = (n_omega + 1) & ~1
-            if v0 is not None:
-                rows.D, rows.v0 = _model_rows(D, v0, B, ld, s, dev)
-            elif D is not None:
+                alpha_rows = (alpha[None, :] * _dev_f64(alpha_scale, dev).reshape(-1, 1)).contiguous()
+        ld = (n_omega + 1) & ~1
+        D_rows = v0_rows = None
+        if v0 is not None:                       # rows built on the device already
+            if D is None or tuple(D.shape) != (B, ld) or v0.shape[0] != B or v0.shape[1] > s:
+                raise ValueError("ready-made model rows must be D[%d, %d] and v0[%d, <= %d]" % (B, ld, B, s))
+            D_rows, v0_rows = _dev_f64(D, dev), zeros(B, s)
+            v0_rows[:, :v0.shape[1]] = _dev_f64(v0, dev)
+        elif D is not None or index is not None:
+            D_rows, v0_rows = zeros(B, ld), zeros(B, s)
+            if D is None:                        # the shared model, with the initial vector of every spectrum's group
+                D_rows[:, :n_omega] = prob.D
+                for q, sel in parts:
+                    v0_rows[sel, :q.n_sv] = q.v0
+            else:                                # one default model per spectrum, v0 in its own group's basis
                 D = _dev_f64(D, dev)
                 if tuple(D.shape) != (B, n_omega):
                     raise ValueError("D must be [%d, %d]" % (B, n_omega))
-                rows.D = torch.zeros((B, ld), dtype=f64, device=dev)
-                rows.v0 = torch.zeros((B, s), dtype=f64, device=dev)
-            else:
-                rows.v0 = torch.stack([q.v0 for q in probs])[index].contiguous()
-                rows.D = torch.zeros((B, ld), dtype=f64, device=dev)
-                rows.D[:, :n_omega] = prob.D
-            for g, q in enumerate(probs):              # projection per group: its own Q, 1/err and row count
-                sel = torch.nonzero(index == g).flatten()
-                if sel.numel() == 0:
-                    continue
-                if D is not None and v0 is None:       # the spectrum's own model, v0 in its group's basis
-                    qb = getattr(q, "base", q)
-                    Dg, vg = per_spectrum_models(qb, D[sel], getattr(qb, "A_init_host", None))
-                    rows.D[sel] = Dg
-                    rows.v0[sel, :qb.n_sv] = vg
-                Gg = G[sel][:, :q.n_tau].contiguous()
-                qq = getattr(q, "base", q)                 # projection in the group's own (unpadded) singular space
-                gg = torch.empty((sel.numel(), qq.n_sv), dtype=f64, device=dev)
-                cg = torch.empty((sel.numel(),), dtype=f64, device=dev)
-                ops.project_data(*_problem_args(qq, alpha, False, lm, chi2_factor), Gg, gg, cg)
-                gt[sel] = 0.0
-                gt[sel, :qq.n_sv] = gg
-                c0[sel] = cg
-        else:
-            if G.shape[1] != prob.n_tau:
-                raise ValueError("G has %d data points, kernel has %d" % (G.shape[1], prob.n_tau))
-            if v0 is not None:                   # rows built on the device already
-                rows.D, rows.v0 = _model_rows(D, v0, B, (n_omega + 1) & ~1, s, dev)
-            elif D is not None:                  # one default model per spectrum, D[B, n_omega]
-                rows.D, rows.v0 = per_spectrum_models(prob, D, getattr(prob, "A_init_host", None))
-                if rows.D.shape[0] != B:
-                    raise ValueError("D has %d rows for %d spectra" % (rows.D.shape[0], B))
-            if sigma is not None:                # Xi_b = Xi / sigma_b, data divided by sigma_b (prob carries err = 1)
-                sg = _dev_f64(sigma, dev).reshape(-1)
-                if sg.numel() != B:
-                    raise ValueError("sigma has %d entries for %d spectra" % (sg.numel(), B))
-                rows.xi = (prob.xi[None, :] / sg[:, None]).contiguous()
-                G = (G / sg[:, None]).contiguous()
-            ops.project_data(*_problem_args(prob, alpha, False, lm, chi2_factor), G, gt, c0)
-        p = _problem_struct(prob, alpha, probability, lm, chi2_factor, rows)
-        pargs = _problem_args(prob, alpha, probability, lm, chi2_factor, rows)
+                D_rows[:, :n_omega] = D
+                for q, sel in parts:
+                    v0_rows[sel, :q.n_sv] = _log_initial_arg(D[sel], q.A_init, q.delta, q.variant) @ q.Vp
+        # ---- launch ----
+        pargs = _problem_args(prob, alpha, lm, chi2_factor, probability, n_sv=s, Vt=Vt, xi=xi, D=D_rows, v0=v0_rows,
+                              vt_index=vt_index, vt_stride=vt_stride, alpha_rows=alpha_rows)
         r = SweepResult()
-        r.alpha = alpha
-        r.n_sv = s
+        r.alpha, r.n_sv, r.problems, r.index, r.alpha_scale = alpha, s, probs, index, alpha_scale
         r.v = torch.empty((B, n_alpha, s), dtype=f64, device=dev) if want_v else None
         r.A = torch.empty((B, n_alpha, n_omega), dtype=f64, device=dev) if want_A else None
         r.chi2 = torch.empty((B, n_alpha), dtype=f64, device=dev)
@@ -582,7 +523,7 @@ def run_sweep(prob, G, alpha_eff, probability=False, lm=None, chi2_factor=1.0, w
         r.n_trial = torch.zeros((B, n_alpha), dtype=i32, device=dev)
         r.n_batch = torch.zeros((B, n_alpha), dtype=i32, device=dev)
         r.phase_cycles = torch.zeros((B, 8), dtype=torch.int64, device=dev) if phase_timers else None
-        ws_bytes = int(lib.mx_sweep_workspace_bytes(ctypes.byref(p), B))
+        ws_bytes = int(prob.lib.mx_sweep_workspace_bytes(ctypes.byref(ops.problem_struct(*pargs)), B))
         if ws_bytes < 0:
             _lib.check(ws_bytes, "mx_sweep_workspace_bytes")
         ws = getattr(prob, "_workspace", None)

@@ -52,7 +52,8 @@ def _f64c(*ts):
             raise ValueError("maxent_b200 operators take contiguous float64 tensors")
 
 
-def _problem(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params):
+def problem_struct(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params):
+    """The MxProblem of the C ABI that the leading arguments of project_data / alpha_sweep describe."""
     if len(dims) != 12 or len(params) != 7:
         raise ValueError("dims must hold 12 integers and params 7 floats (see maxent_b200/ops.py)")
     if vt_index is not None and (vt_index.dtype != torch.int32 or not vt_index.is_contiguous()):
@@ -66,7 +67,7 @@ def _problem(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params)
 
 
 def _project_data(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params, G, gt, c0):
-    p = _problem(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params)
+    p = problem_struct(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params)
     _f64c(G, gt, c0)
     with torch.cuda.device(G.device):
         _lib.check(_lib.load().mx_project_data(ctypes.byref(p), _ptr(G), int(G.shape[0]), _ptr(gt), _ptr(c0),
@@ -75,7 +76,7 @@ def _project_data(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, pa
 
 def _alpha_sweep(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params, gt, c0, v, A, chi2, S, Q, logp,
                  n_iter, n_qeval, n_solve, status, n_trial, n_batch, phase_cycles, workspace):
-    p = _problem(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params)
+    p = problem_struct(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params)
     _f64c(gt, c0, v, A, chi2, S, Q, logp)
     out = _lib.MxSweepOut(_ptr(v), _ptr(A), _ptr(chi2), _ptr(S), _ptr(Q), _ptr(logp), _ptr(n_iter), _ptr(n_qeval),
                           _ptr(n_solve), _ptr(status), _ptr(n_trial), _ptr(n_batch), _ptr(phase_cycles))

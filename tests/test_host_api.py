@@ -344,6 +344,69 @@ def test_batched_front_end_accepts_a_levenberg_minimizer():
     assert isinstance(mb.BatchedTauMaxEnt(minimizer=engine.LMParams(nu=1.5)).minimizer, engine.LMParams)
 
 
+def test_batched_whitening_groups_are_planned_on_the_whole_batch(monkeypatch):
+    """BatchedTauMaxEnt numbers the whitening groups of err[B, n_tau] in the sorted order of the vectors, those of
+    cov[B, n, n] in the order of first appearance and those of set_error_groups as given.  A run that leaves a spectrum
+    below G_threshold out of the launch keeps the groups of the whole batch, so the next run of the same job gives every
+    spectrum its own error vector again.  SharedProblem and run_sweep are replaced by recorders: no device is used."""
+    import torch
+    import maxent_b200 as mb
+    from maxent_b200 import batched, engine
+    n_tau = 4
+    job = mb.BatchedTauMaxEnt(scale_alpha=None)
+    job.set_G_tau_data(np.linspace(0, 1, n_tau), np.ones((1, n_tau)))
+    vec = np.array([3e-3, 1e-3, 2e-3])
+    which = np.array([0, 1, 2, 1])
+    job.set_error(np.repeat(vec[which][:, None], n_tau, axis=1))
+    mode, index, specs = job._error_plan(4)
+    assert mode == "groups" and index.tolist() == [2, 0, 1, 0] and [s[1][0] for s in specs] == [1e-3, 2e-3, 3e-3]
+    job.set_error_groups(vec[:, None] * np.ones(n_tau), which)
+    mode, index, specs = job._error_plan(4)
+    assert mode == "groups" and index.tolist() == which.tolist() and [s[1][0] for s in specs] == vec.tolist()
+    C = [np.diag(np.full(n_tau, c)) for c in (4.0, 1.0, 9.0)]
+    job.set_cov(np.stack([C[k] for k in which]))
+    mode, index, specs = job._error_plan(4)
+    assert mode == "groups" and index.tolist() == which.tolist() and [s[1][0] for s in specs] == [2.0, 1.0, 3.0]
+
+    class Problem(object):
+        def __init__(self, K, err, *args, **kwargs):
+            self.err = np.atleast_1d(np.asarray(err, dtype=np.float64))
+            self.n_tau, self.n_omega, self.n_sv, self.device, self.U, self.S, self.V = n_tau, 3, 2, torch.device("cpu"), 0, 0, 0
+
+    def run_sweep(prob, G, alpha, groups=None, **kwargs):
+        B, n_alpha = int(G.shape[0]), len(alpha)
+        r = engine.SweepResult()
+        for name in ("chi2", "S", "Q", "logp"):
+            setattr(r, name, torch.zeros((B, n_alpha), dtype=torch.float64))
+        for name in ("n_iter", "n_qeval", "n_solve", "status", "n_trial", "n_batch"):
+            setattr(r, name, torch.zeros((B, n_alpha), dtype=torch.int32))
+        r.alpha_index = torch.zeros((B, 5), dtype=torch.int32)
+        r.A, r.A_out = torch.zeros((B, n_alpha, 3), dtype=torch.float64), torch.zeros((B, 5, 3), dtype=torch.float64)
+        r.v = None
+        r.alpha, r.n_sv, r.phase_cycles, r.alpha_scale = torch.as_tensor(alpha), 2, None, None
+        r.problems, r.index = groups
+        launched.append([r.problem(b).err[0] for b in range(B)])
+        return r
+
+    base = Problem(np.ones((n_tau, 3)), 1.0)
+    monkeypatch.setattr(engine, "SharedProblem", Problem)
+    monkeypatch.setattr(engine, "run_sweep", run_sweep)
+    monkeypatch.setattr(batched.BatchedTauMaxEnt, "prepare", lambda self: base)
+    job._K_dev, job._D_host = torch.ones((n_tau, 3), dtype=torch.float64), np.ones(3)
+    job.omega, job.alpha_mesh = batched.DataOmegaMesh(np.linspace(-1, 1, 3)), [2.0, 1.0]
+    job.set_error(np.repeat(vec[which][:, None], n_tau, axis=1))
+    G = torch.ones((4, n_tau), dtype=torch.float64)
+    G[0] = 0.0                                       # the only spectrum of its group is below G_threshold
+    launched = []
+    res = job.run_device(G, skip_small=True)
+    assert launched == [[1e-3, 2e-3, 1e-3]]
+    assert [res.problem(b).err[0] for b in (1, 2, 3)] == [1e-3, 2e-3, 1e-3]
+    launched = []
+    res = job.run_device(torch.ones((4, n_tau), dtype=torch.float64), skip_small=True)
+    assert launched == [vec[which].tolist()]
+    assert [res.problem(b).err[0] for b in range(4)] == vec[which].tolist()
+
+
 def test_meshes_and_default_model_match_the_reference_exactly():
     """Tier T0 (SURVEY.md 8(c)): omega meshes with their integration weights, alpha meshes and the flat default model
     are the reference's arrays (tests/golden/g0_meshes.npz, written by oracle/make_golden.py from the real
