@@ -28,11 +28,6 @@ extern "C" {
 #define MX_MAX_NSV         256   /* singular-space dimension the fused path supports: up to 80 with every matrix in
                                     * shared memory and registers, 81..256 with Z, J and the factors in the workspace */
 
-/* sweep engines (MxProblem.engine) */
-#define MX_ENGINE_AUTO       0   /* = MX_ENGINE_SPECTRUM_CTA */
-#define MX_ENGINE_LOCKSTEP   1   /* retired (round-1 lock-step engine): requesting it returns MX_ERR_UNSUPPORTED */
-#define MX_ENGINE_SPECTRUM_CTA 2 /* one spectrum per CTA, speculative damping batches (csrc/mx_sweep2.cuh)    */
-
 /* MxProblem.per_spectrum_model bits */
 #define MX_PER_SPECTRUM_MODEL 1
 #define MX_PER_SPECTRUM_XI    2
@@ -82,7 +77,6 @@ typedef struct {
     int32_t n_alpha;
     int32_t variant;          /* MX_VARIANT_*                                                */
     int32_t want_probability; /* NormalLogProbability (probabilities.py:76-85)               */
-    int32_t engine;           /* MX_ENGINE_*                                                 */
     int32_t per_spectrum_model; /* bit mask.  MX_PER_SPECTRUM_MODEL: D[B, ldD], v0[B, n_sv] instead of D[n_omega], v0[n_sv],
                                * row stride ldD = n_omega rounded up to an even number (16-byte aligned rows)
                                * (PoormanMaxEnt off-diagonals, python/elementwise_maxent.py:633-652).
@@ -191,10 +185,9 @@ int mx_alpha_sweep(const MxProblem* p, const double* gt, const double* c0, int32
 /* Device workspace mx_alpha_sweep needs for this problem and batch size on the current device (<0: MX_ERR_*). */
 int64_t mx_sweep_workspace_bytes(const MxProblem* p, int32_t B);
 
-/* Introspection for tests / DESIGN.md: engine actually used for (n_sv, engine), spectra marched per CTA,
- * dynamic shared memory and threads per CTA.  Needs no device. */
-int mx_sweep_config(int32_t n_sv, int32_t engine, int32_t* engine_used, int32_t* spectra_per_cta,
-                    int32_t* smem_bytes, int32_t* threads);
+/* Introspection for tests / DESIGN.md: dynamic shared memory and threads per CTA of the sweep kernel for n_sv
+ * (one spectrum per CTA, csrc/mx_sweep2.cuh).  Needs no device. */
+int mx_sweep_config(int32_t n_sv, int32_t* smem_bytes, int32_t* threads);
 
 /* Analyzer reductions (python/analyzers/*.py) for B spectra:
  * alpha_index[B, MX_N_ANALYZERS] (-1 = not available), A_out[B, MX_N_ANALYZERS, n_omega] (may be NULL),

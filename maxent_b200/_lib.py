@@ -12,7 +12,6 @@ LIB_PATH = os.environ.get("MAXENT_B200_LIB") or os.path.join(HERE, "libmaxent_b2
 
 MX_OK = 0
 MX_MAX_NSV = 256
-ENGINE_AUTO, ENGINE_LOCKSTEP, ENGINE_SPECTRUM_CTA = 0, 1, 2
 VARIANTS = {"normal": 0, "plusminus": 1, "bryan": 2}
 AN_LINEFIT, AN_CHI2CURV, AN_ENTROPY, AN_CLASSIC, AN_BRYAN = range(5)
 N_ANALYZERS = 5
@@ -39,7 +38,7 @@ class MxLMParams(ctypes.Structure):
 class MxProblem(ctypes.Structure):
     _fields_ = [("n_tau", ctypes.c_int32), ("n_omega", ctypes.c_int32), ("n_sv", ctypes.c_int32),
                 ("n_alpha", ctypes.c_int32), ("variant", ctypes.c_int32), ("want_probability", ctypes.c_int32),
-                ("engine", ctypes.c_int32), ("per_spectrum_model", ctypes.c_int32), ("chi2_factor", ctypes.c_double),
+                ("per_spectrum_model", ctypes.c_int32), ("chi2_factor", ctypes.c_double),
                 ("Vt", c_dp), ("Qw", c_dp), ("Qo", c_dp), ("sqrtw", c_dp), ("xi", c_dp), ("D", c_dp),
                 ("delta", c_dp), ("alpha", c_dp), ("v0", c_dp), ("lm", MxLMParams), ("vt_index", c_dp),
                 ("vt_stride", ctypes.c_int64)]
@@ -69,9 +68,7 @@ SYMBOLS = [
     ("mx_alpha_sweep", ctypes.c_int, [ctypes.POINTER(MxProblem), c_dp, c_dp, ctypes.c_int32,
                                       ctypes.POINTER(MxSweepOut), c_dp, ctypes.c_int64, c_dp]),
     ("mx_sweep_workspace_bytes", ctypes.c_int64, [ctypes.POINTER(MxProblem), ctypes.c_int32]),
-    ("mx_sweep_config", ctypes.c_int, [ctypes.c_int32, ctypes.c_int32, ctypes.POINTER(ctypes.c_int32),
-                                       ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32),
-                                       ctypes.POINTER(ctypes.c_int32)]),
+    ("mx_sweep_config", ctypes.c_int, [ctypes.c_int32, ctypes.POINTER(ctypes.c_int32), ctypes.POINTER(ctypes.c_int32)]),
     ("mx_analyze", ctypes.c_int, [c_dp, c_dp, c_dp, c_dp, c_dp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32,
                                   ctypes.c_double, ctypes.c_int32, ctypes.c_int32, c_dp, c_dp, c_dp, c_dp]),
     ("mx_poorman_models", ctypes.c_int, [c_dp, ctypes.c_int32, c_dp, ctypes.c_int32, c_dp, ctypes.c_double, c_dp, c_dp,
@@ -104,9 +101,8 @@ def check(rc, what):
         raise MaxEntLibraryError("%s failed: %s (code %d)" % (what, _ERR.get(rc, "unknown"), rc))
 
 
-def sweep_config(n_sv, engine=ENGINE_AUTO):
+def sweep_config(n_sv):
     lib = load()
-    e, t, sm, th = ctypes.c_int32(), ctypes.c_int32(), ctypes.c_int32(), ctypes.c_int32()
-    check(lib.mx_sweep_config(n_sv, engine, ctypes.byref(e), ctypes.byref(t), ctypes.byref(sm), ctypes.byref(th)),
-          "mx_sweep_config")
-    return dict(engine=e.value, spectra_per_cta=t.value, smem_bytes=sm.value, threads=th.value)
+    sm, th = ctypes.c_int32(), ctypes.c_int32()
+    check(lib.mx_sweep_config(n_sv, ctypes.byref(sm), ctypes.byref(th)), "mx_sweep_config")
+    return dict(smem_bytes=sm.value, threads=th.value)

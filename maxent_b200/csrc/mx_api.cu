@@ -417,17 +417,14 @@ static int fill_args(const MxProblem* p, SweepArgs& a) {
     return MX_OK;
 }
 
-int mx_sweep_config(int32_t n_sv, int32_t engine, int32_t* engine_used, int32_t* spectra_per_cta, int32_t* smem_bytes,
-                    int32_t* threads) {
+int mx_sweep_config(int32_t n_sv, int32_t* smem_bytes, int32_t* threads) {
     SweepArgs a = {};
     a.n_sv = n_sv;
     a.B = 1;
     a.conv_absq = -1.0;
-    int t = 0, sm = 0, eng = 0;
-    const int rc = dispatch_sweep(a, nullptr, true, engine, &eng, &t, &sm, nullptr);
+    int sm = 0;
+    const int rc = dispatch_sweep(a, nullptr, true, &sm, nullptr);
     if (rc != MX_OK) return rc;
-    if (engine_used) *engine_used = eng;
-    if (spectra_per_cta) *spectra_per_cta = t;
     if (smem_bytes) *smem_bytes = sm;
     if (threads) *threads = sweep_threads();
     return MX_OK;
@@ -435,30 +432,30 @@ int mx_sweep_config(int32_t n_sv, int32_t engine, int32_t* engine_used, int32_t*
 
 static const int64_t WS_HEADER = 256;     // bytes reserved for the work counter in front of the scratch rows
 
-// persistent CTAs the sweep would be launched with (what the workspace is sized for)
-static int sweep_grid(const MxProblem* p, int32_t B, int* grid) {
-    SweepArgs a = {};
-    a.n_sv = p->n_sv;
+// fills a for a sweep of B spectra of p and finds the persistent CTAs it would be launched with (what the workspace is
+// sized for)
+static int sweep_grid(const MxProblem* p, int32_t B, SweepArgs& a, int* grid) {
+    int rc = fill_args(p, a);
+    if (rc != MX_OK) return rc;
     a.B = B > 0 ? B : 1;
-    a.per_spec = (p->per_spectrum_model & MX_PER_SPECTRUM_MODEL) ? 1 : 0;
-    a.per_spec_xi = (p->per_spectrum_model & MX_PER_SPECTRUM_XI) ? 1 : 0;
-    a.per_spec_alpha = (p->per_spectrum_model & MX_PER_SPECTRUM_ALPHA) ? 1 : 0;
-    a.marquardt = p->lm.marquardt ? 1 : 0;
-    a.variant = p->variant;
-    a.conv_absq = p->lm.conv_abs_change;
-    int eng = 0;
     *grid = 0;
-    const int rc = dispatch_sweep(a, nullptr, true, p->engine, &eng, nullptr, nullptr, grid);
+    rc = dispatch_sweep(a, nullptr, true, nullptr, grid);
     if (rc != MX_OK) return rc;
     return *grid > 0 ? MX_OK : MX_ERR_NO_DEVICE;
 }
 
+// work counter + scratch rows + wide slices of a sweep of p on `grid` CTAs
+static int64_t sweep_workspace_bytes(const MxProblem* p, int grid) {
+    return WS_HEADER + 8 * sweep_scratch_doubles(p->n_sv, p->n_omega, p->variant, grid);
+}
+
 int64_t mx_sweep_workspace_bytes(const MxProblem* p, int32_t B) {
     if (!p || B < 0) return MX_ERR_BAD_ARG;
+    SweepArgs a = {};
     int grid = 0;
-    const int rc = sweep_grid(p, B, &grid);
+    const int rc = sweep_grid(p, B, a, &grid);
     if (rc != MX_OK) return rc;
-    return WS_HEADER + 8 * sweep_scratch_doubles(p->n_sv, p->n_omega, p->variant, grid);
+    return sweep_workspace_bytes(p, grid);
 }
 
 int mx_alpha_sweep(const MxProblem* p, const double* gt, const double* c0, int32_t B, const MxSweepOut* out,
@@ -467,14 +464,12 @@ int mx_alpha_sweep(const MxProblem* p, const double* gt, const double* c0, int32
     if (!p || !gt || !c0 || !out || !workspace || B < 0) return MX_ERR_BAD_ARG;
     if (!out->chi2 || !out->S || !out->Q) return MX_ERR_BAD_ARG;
     SweepArgs a = {};
-    int rc = fill_args(p, a);
-    if (rc != MX_OK) return rc;
     int grid = 0;
-    rc = sweep_grid(p, B, &grid);
+    const int rc = sweep_grid(p, B, a, &grid);
     if (rc != MX_OK) return rc;
-    const int64_t need = WS_HEADER + 8 * sweep_scratch_doubles(p->n_sv, p->n_omega, p->variant, grid);
-    if (workspace_bytes < need || (reinterpret_cast<uintptr_t>(workspace) & 15) != 0) return MX_ERR_BAD_ARG;
-    a.B = B; a.gt = gt; a.c0 = c0;
+    if (workspace_bytes < sweep_workspace_bytes(p, grid) || (reinterpret_cast<uintptr_t>(workspace) & 15) != 0)
+        return MX_ERR_BAD_ARG;
+    a.gt = gt; a.c0 = c0;
     a.o_v = out->v; a.o_A = out->A; a.o_chi2 = out->chi2; a.o_S = out->S; a.o_Q = out->Q; a.o_logp = out->logp;
     a.o_niter = out->n_iter; a.o_nq = out->n_qeval; a.o_ns = out->n_solve; a.o_status = out->status;
     a.o_ntrial = out->n_trial; a.o_nbatch = out->n_batch; a.o_phase = reinterpret_cast<long long*>(out->phase_cycles);
@@ -483,7 +478,7 @@ int mx_alpha_sweep(const MxProblem* p, const double* gt, const double* c0, int32
     a.wide_stride = sweep_wide_stride(p->n_sv);         // the slices of the wide instantiations follow the scratch rows
     a.wide = a.wide_stride ? a.scratch + sweep_rows_doubles(p->n_omega, p->variant, grid) : nullptr;
     if (cudaMemsetAsync(workspace, 0, WS_HEADER, (cudaStream_t)stream) != cudaSuccess) return MX_ERR_CUDA;
-    return dispatch_sweep(a, (cudaStream_t)stream, false, p->engine, nullptr, nullptr, nullptr, nullptr);
+    return dispatch_sweep(a, (cudaStream_t)stream, false, nullptr, nullptr);
 }
 
 int mx_analyze(const double* alpha, const double* chi2, const double* S, const double* logp, const double* A,

@@ -31,19 +31,14 @@ int64_t sweep_scratch_doubles(int n_sv, int n_omega, int variant, int grid) {
     return sweep_rows_doubles(n_omega, variant, grid) + (int64_t)grid * sweep_wide_stride(n_sv);
 }
 
-int dispatch_sweep(SweepArgs& a, cudaStream_t stream, bool query, int engine, int* o_engine, int* o_t, int* o_smem, int* o_grid) {
+int dispatch_sweep(SweepArgs& a, cudaStream_t stream, bool query, int* o_smem, int* o_grid) {
     const int s = a.n_sv;
     if (s < 1) return MX_ERR_BAD_ARG;
     int pk = (s * (s + 1)) / 2;
     pk = (pk + 1) & ~1;
     a.pk = pk;
     if (s > MX_MAX_NSV) return MX_ERR_UNSUPPORTED;
-    const int nt = sweep_tiles(s);
-    if (engine == 0) engine = MX_ENGINE_SPECTRUM_CTA;
-    if (engine != MX_ENGINE_SPECTRUM_CTA) return MX_ERR_UNSUPPORTED;       // the lock-step engine of round 1 is retired
-    if (o_engine) *o_engine = engine;
-    if (o_t) *o_t = 1;
-    switch (nt) {
+    switch (sweep_tiles(s)) {
         case 4: return mx2::sweep2_nt4(a, stream, query, o_smem, o_grid);
         case 5: return mx2::sweep2_nt5(a, stream, query, o_smem, o_grid);
         case 6: return mx2::sweep2_nt6(a, stream, query, o_smem, o_grid);

@@ -1,7 +1,7 @@
 // Fused MaxEnt alpha sweep for sm_100a (B200), "spectrum per CTA".
 //
-// One CTA of MX_NWARP warps (8; 4 is supported) owns one spectrum at a time (persistent CTAs, atomic work counter, as
-// many CTAs per SM as registers and shared memory allow: two at 8 warps) and runs the whole alpha mesh for it.
+// One CTA of 8 warps owns one spectrum at a time (persistent CTAs, atomic work counter, as many CTAs per SM as
+// registers and shared memory allow: two) and runs the whole alpha mesh for it.
 // Round 2 measured the alternatives on B200 (profiles/r02_ab_*.log): four 4-warp CTAs per SM are 10 % slower, three
 // 4-warp CTAs at 168 registers 3 % slower than two 8-warp CTAs -- the FP64 pipe is 62-68 % busy in all three, so the
 // idle third is not a matter of how the warps are grouped.  The Levenberg-Marquardt iteration of the reference
@@ -42,14 +42,8 @@ using mx::SweepArgs;
 using mx::dmma;
 using mx::tile_off;
 
-#ifndef MX_NWARP
-#define MX_NWARP 8
-#endif
-#ifndef MX_CTAS_PER_SM          // CTAs per SM the kernel is compiled for: register cap = 64K / (CTAs x threads)
-#define MX_CTAS_PER_SM (MX_NWARP == 4 ? 4 : 2)
-#endif
-constexpr int NWARP = MX_NWARP;
-static_assert(NWARP == 4 || NWARP == 8, "the reduction trees are written for 4 or 8 warps");
+constexpr int NWARP = 8;        // the fixed-order reduction trees over the warps are written for 8
+constexpr int CTAS_PER_SM = 2;  // CTAs per SM the kernel is compiled for: register cap = 64K / (CTAs x threads)
 constexpr int NTHR = NWARP * 32;
 constexpr int NKG = NWARP / 2;  // k-groups of the H-pass (two warps -- the two halves of the triangle -- per group)
 constexpr int CH = NWARP;       // k-tiles (8 omega rows each) per staged chunk = one per warp in the T-pass, two per k-group in the H-pass
@@ -143,12 +137,10 @@ __host__ __device__ constexpr int tri(int I, int J) { return I * (I + 1) / 2 + J
 // ------------------------------------------------------------------------------------------
 // sizes of the "lean" blocked Cholesky (see below): how many tiles of the factor a warp parks in shared memory
 // ------------------------------------------------------------------------------------------
-#ifndef MX_LEAN_RTILES
-#define MX_LEAN_RTILES 10       // strictly-lower tiles of the factor a warp keeps in registers
-#endif
+constexpr int LEAN_RTILES = 10;    // strictly-lower tiles of the factor a warp keeps in registers
 __host__ __device__ constexpr int lean_nsm(int NT) {
     int nsm = 0;
-    while (nsm < NT && (NT - 1 - nsm) * (NT - nsm) / 2 > MX_LEAN_RTILES) ++nsm;
+    while (nsm < NT && (NT - 1 - nsm) * (NT - nsm) / 2 > LEAN_RTILES) ++nsm;
     return nsm;
 }
 __host__ __device__ constexpr int lean_nsmt(int NT) {          // strictly-lower tiles of the factor a warp parks in shared memory
@@ -171,26 +163,21 @@ struct Lean {
 };
 
 // Staging buffers of the V' stream: at least two (one being consumed, one in flight), and enough area for what the
-// ring is reused for between passes: Zfull (NT x NT tiles), the parked Cholesky tiles of every warp, the per-warp y
-// partials of the T-pass.  MX_NST_EXTRA adds stages (deeper prefetch) when the CTAs-per-SM target leaves room.
-#ifndef MX_NST_EXTRA
-#define MX_NST_EXTRA 0
-#endif
+// ring is reused for between passes: Zfull (NT x NT tiles), the parked Cholesky tiles of every solving warp, the
+// per-warp y partials of the T-pass.
 // warps that factorise at the same time: all of them up to 7 tiles; beyond that every warp parks so many tiles that
 // a full house would cost the second CTA per SM, so half the warps solve in twice the rounds
 __host__ __device__ constexpr int solver_warps(int NT) { return NT <= 7 ? NWARP : NWARP / 2; }
 __host__ __device__ constexpr int stage_count(int NT) {
     int need = NT * NT;                                                          // in 8x8 tiles
-#ifndef MX_LEAN_SPILLOVER           // the parked tiles may run past the ring into a few KB of their own (STAGE_AREA)
     if (solver_warps(NT) * lean_nsmt(NT) > need) need = solver_warps(NT) * lean_nsmt(NT);
-#endif
     if (NWARP * NT > need) need = NWARP * NT;
     // partial Z tiles of the H-pass: Zfull + (NKG - 1) triangles, minus what J and the trial vectors behind the ring hold
     const int hneed = NT * NT + (NKG - 2) * (NT * (NT + 1) / 2) - 2 * NT;
     if (hneed > need) need = hneed;
     int nst = (need + CH * NT - 1) / (CH * NT);
     if (nst < 2) nst = 2;
-    return nst + MX_NST_EXTRA;
+    return nst;
 }
 
 // ------------------------------------------------------------------------------------------
@@ -1066,12 +1053,12 @@ __device__ __forceinline__ void hpass_body(const Pipe<NT>& pipe, const double* _
 // ------------------------------------------------------------------------------------------
 // the kernel
 // ------------------------------------------------------------------------------------------
-// CTAs per SM the instantiation is compiled for: the target (MX_CTAS_PER_SM), or what its shared memory allows
+// CTAs per SM the instantiation is compiled for: the target (CTAS_PER_SM), or what its shared memory allows
 template <int NT>
 __host__ __device__ constexpr int ctas_per_sm() {
     if (is_wide(NT)) return 1;                // the block accumulators of the wide H-pass need the full register file
     int n = (228 * 1024) / (Lay<NT>::total * (int)sizeof(double) + 1024);
-    if (n > MX_CTAS_PER_SM) n = MX_CTAS_PER_SM;
+    if (n > CTAS_PER_SM) n = CTAS_PER_SM;
     return n < 1 ? 1 : n;
 }
 
@@ -1248,9 +1235,8 @@ __global__ void __launch_bounds__(NTHR, ctas_per_sm<NT>()) sweep2_kernel(const S
         for (int i = tid; i < MAXB * SP; i += NTHR) {      // fixed-order tree over the warps (deterministic sums)
             const int b = i / SP, j = i - b * SP;
             const double* y0 = yred + b * SP + j;
-            double t = (y0[0 * 8 * SP] + y0[1 * 8 * SP]) + (y0[2 * 8 * SP] + y0[3 * 8 * SP]);
-            if constexpr (NWARP == 8) t += (y0[4 * 8 * SP] + y0[5 * 8 * SP]) + (y0[6 * 8 * SP] + y0[7 * 8 * SP]);
-            sm[LY::o_yb + i] = t;
+            sm[LY::o_yb + i] = ((y0[0 * 8 * SP] + y0[1 * 8 * SP]) + (y0[2 * 8 * SP] + y0[3 * 8 * SP]))
+                             + ((y0[4 * 8 * SP] + y0[5 * 8 * SP]) + (y0[6 * 8 * SP] + y0[7 * 8 * SP]));
         }
         __syncthreads();
         for (int u = warp; u < nuniq; u += NWARP) {        // chi2 = |Xi y - g~|^2 + c0  (functions.py:358-360 in singular space)
@@ -1261,8 +1247,7 @@ __global__ void __launch_bounds__(NTHR, ctas_per_sm<NT>()) sweep2_kernel(const S
             }
             c2 = warp_sum(c2) + ctl.c0;
             const double* sr = sm + LY::o_sred + u;
-            double S = (sr[0] + sr[8]) + (sr[16] + sr[24]);
-            if constexpr (NWARP == 8) S += (sr[32] + sr[40]) + (sr[48] + sr[56]);
+            const double S = ((sr[0] + sr[8]) + (sr[16] + sr[24])) + ((sr[32] + sr[40]) + (sr[48] + sr[56]));
             if (lane == 0) {
                 ctl.uchi2[u] = c2; ctl.uS[u] = S;
                 ctl.uQ[u] = ctl.ufail[u] ? nan("") : 0.5 * c2 * a.eta - ctl.alpha * S;   // maxent_cost_function.py:82

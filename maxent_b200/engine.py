@@ -52,7 +52,7 @@ class SharedProblem(object):
     this rotation because mu*1 is."""
 
     def __init__(self, K, err, D, delta, variant="normal", reduce_singular_space=1.e-14, device=None,
-                 svd="jacobi", A_init=None, max_nsv=None, engine=0, rank_floor=5.e-16, usv=None,
+                 svd="jacobi", A_init=None, max_nsv=None, rank_floor=5.e-16, usv=None,
                  orthonormal_U=True):
         """``usv`` = (U, S, V) already truncated by the caller (a ``kernels.KernelSVD`` after
         ``reduce_singular_space``); ``orthonormal_U=False`` when U was rotated by a non-square T
@@ -144,8 +144,7 @@ class SharedProblem(object):
             self.A_init = None if A_init is None else _dev_f64(A_init, dev)
             self.v0 = (self.Vp.transpose(0, 1) @ _log_initial_arg(self.D, self.A_init, self.delta, variant)).contiguous()
             self.Vt = _layout_V(self.lib, self.Vp)
-            self.engine = int(engine)
-            self.config = _lib.sweep_config(s, self.engine)
+            self.config = dict(_lib.sweep_config(s), spectra_per_cta=1)   # bench.py reports spectra_per_cta
 
     def _reorthonormalize(self, Q):
         """Columns of Q made orthonormal in order, on the device in one launch (mx_gram_schmidt_rows)."""
@@ -334,7 +333,7 @@ def _problem_args(prob, alpha, lm, chi2_factor, probability=False, n_sv=None, Vt
              | (_lib.PER_SPECTRUM_VT if vt_index is not None else 0)
              | (_lib.PER_SPECTRUM_ALPHA if alpha_rows is not None else 0))
     dims = [prob.n_tau, prob.n_omega, prob.n_sv if n_sv is None else n_sv, int(alpha.numel()), _lib.VARIANTS[prob.variant],
-            int(bool(probability)), prob.engine, flags, int(lm.maxiter), int(lm.miniter), int(lm.marquardt), int(vt_stride)]
+            int(bool(probability)), flags, int(lm.maxiter), int(lm.miniter), int(lm.marquardt), int(vt_stride)]
     params = [float(chi2_factor), float(lm.mu0), float(lm.nu), float(lm.max_mu), float(lm.conv_max_derivative),
               float(lm.conv_rel_change), float(lm.conv_abs_change)]
     return (prob.Vt if Vt is None else Vt, prob.Qw, prob.Q, prob.sqrtw, prob.xi if xi is None else xi,

@@ -20,8 +20,8 @@ import torch
 
 from . import _lib
 
-# dims  = [n_tau, n_omega, n_sv, n_alpha, variant, want_probability, engine, per_spectrum_model, maxiter, miniter,
-#          marquardt, vt_stride]
+# dims  = [n_tau, n_omega, n_sv, n_alpha, variant, want_probability, per_spectrum_model, maxiter, miniter, marquardt,
+#          vt_stride]
 # param = [chi2_factor, mu0, nu, max_mu, conv_max_derivative, conv_rel_change, conv_abs_change]
 _PROBLEM = ("Tensor Vt, Tensor Qw, Tensor Qo, Tensor sqrtw, Tensor xi, Tensor D, Tensor delta, Tensor alpha, "
             "Tensor v0, Tensor? vt_index, int[] dims, float[] params")
@@ -54,16 +54,16 @@ def _f64c(*ts):
 
 def problem_struct(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params):
     """The MxProblem of the C ABI that the leading arguments of project_data / alpha_sweep describe."""
-    if len(dims) != 12 or len(params) != 7:
-        raise ValueError("dims must hold 12 integers and params 7 floats (see maxent_b200/ops.py)")
+    if len(dims) != 11 or len(params) != 7:
+        raise ValueError("dims must hold 11 integers and params 7 floats (see maxent_b200/ops.py)")
     if vt_index is not None and (vt_index.dtype != torch.int32 or not vt_index.is_contiguous()):
         raise ValueError("vt_index must be a contiguous int32 tensor")
     _f64c(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0)
-    lm = _lib.MxLMParams(int(dims[8]), int(dims[9]), float(params[1]), float(params[2]), float(params[3]),
-                         float(params[4]), float(params[5]), float(params[6]), int(dims[10]), 0)
+    lm = _lib.MxLMParams(int(dims[7]), int(dims[8]), float(params[1]), float(params[2]), float(params[3]),
+                         float(params[4]), float(params[5]), float(params[6]), int(dims[9]), 0)
     return _lib.MxProblem(int(dims[0]), int(dims[1]), int(dims[2]), int(dims[3]), int(dims[4]), int(dims[5]),
-                          int(dims[6]), int(dims[7]), float(params[0]), _ptr(Vt), _ptr(Qw), _ptr(Qo), _ptr(sqrtw),
-                          _ptr(xi), _ptr(D), _ptr(delta), _ptr(alpha), _ptr(v0), lm, _ptr(vt_index), int(dims[11]))
+                          int(dims[6]), float(params[0]), _ptr(Vt), _ptr(Qw), _ptr(Qo), _ptr(sqrtw),
+                          _ptr(xi), _ptr(D), _ptr(delta), _ptr(alpha), _ptr(v0), lm, _ptr(vt_index), int(dims[10]))
 
 
 def _project_data(Vt, Qw, Qo, sqrtw, xi, D, delta, alpha, v0, vt_index, dims, params, G, gt, c0):

@@ -61,17 +61,16 @@ def test_struct_layout_matches_c(tmp_path):
     assert int(out["MX_N_ANALYZERS"]) == _lib.N_ANALYZERS
 
 
-def test_introspection_calls_without_gpu(lib):
+def test_host_introspection_without_gpu(lib):
     """The two pure-host entry points work without a device; version string names the architecture."""
     assert b"sm_100a" in lib.mx_version()
     from maxent_b200 import _lib
     for s in (8, 32, 47, 52, 64):
         cfg = _lib.sweep_config(s)
-        assert cfg["engine"] == _lib.ENGINE_SPECTRUM_CTA and cfg["spectra_per_cta"] == 1 and cfg["threads"] == 256
+        assert cfg["threads"] == 256
         assert 2 * (cfg["smem_bytes"] + 1024) <= 228 * 1024  # two 8-warp CTAs per SM
-    assert lib.mx_sweep_config(52, _lib.ENGINE_LOCKSTEP, None, None, None, None) == -2    # retired engine
-    e = ctypes.c_int32()
-    assert lib.mx_sweep_config(_lib.MX_MAX_NSV + 1, 0, ctypes.byref(e), None, None, None) == -2
+    sm = ctypes.c_int32()
+    assert lib.mx_sweep_config(_lib.MX_MAX_NSV + 1, ctypes.byref(sm), None) == -2
     n = lib.mx_layout_V_size(1000, 52)
     assert n == 125 * 7 * 64
     assert lib.mx_layout_V_size(1000, 0) < 0
@@ -114,5 +113,5 @@ def test_torch_operators_registered_cuda_only():
         ops.analyze(t[0], t, t, None, None, 0.2, 0, False, torch.zeros((1, 5), dtype=torch.int32), None, None)
     z = torch.zeros(4, dtype=torch.float64)
     with pytest.raises(NotImplementedError):
-        ops.project_data(z, z, z, z, z, z, z, z, z, None, [2, 2, 2, 1, 0, 0, 0, 0, 10, 0, 0, 0], [1.0, 1e-18, 1.3, 1e20, 1e-4, 1e-16, -1.0],
+        ops.project_data(z, z, z, z, z, z, z, z, z, None, [2, 2, 2, 1, 0, 0, 0, 10, 0, 0, 0], [1.0, 1e-18, 1.3, 1e20, 1e-4, 1e-16, -1.0],
                          t, t, z)

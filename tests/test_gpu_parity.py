@@ -332,7 +332,7 @@ def test_analyzers_vs_oracle_on_mock_results(torch_cuda):
         assert idx[b, 0] == mo.analyze_linefit(alpha, chi2n[b], A[b], 0)["alpha_index"], b
 
 
-def test_edge_cases(torch_cuda):
+def test_sweep_edge_cases(torch_cuda):
     """Empty batch, n_sv beyond the fused path, bad nu."""
     torch = torch_cuda
     from maxent_b200 import engine, _lib
@@ -345,8 +345,8 @@ def test_edge_cases(torch_cuda):
         engine.LMParams(nu=1.0)
     lib = _lib.load()
     assert lib.mx_layout_V_size(40, _lib.MX_MAX_NSV + 1) < 0
-    e, t, sm, th = ctypes.c_int32(), ctypes.c_int32(), ctypes.c_int32(), ctypes.c_int32()
-    assert lib.mx_sweep_config(_lib.MX_MAX_NSV + 1, 0, ctypes.byref(e), ctypes.byref(t), ctypes.byref(sm), ctypes.byref(th)) == -2
+    sm, th = ctypes.c_int32(), ctypes.c_int32()
+    assert lib.mx_sweep_config(_lib.MX_MAX_NSV + 1, ctypes.byref(sm), ctypes.byref(th)) == -2
 
 
 # ----------------------------------------------------------------------------------------------

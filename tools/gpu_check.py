@@ -10,14 +10,13 @@ np.set_printoptions(linewidth=220, precision=2)
 names = sys.argv[1:] or ["g2_synth_200x100.npz", "g3_plusminus_offdiag.npz", "g4_bryan_200x100.npz",
                          "g1_semicircular_prob.npz", "g5_config1_cut1e-11.npz"]
 svd = os.environ.get("MX_SVD", "jacobi")
-engine_id = int(os.environ.get("MX_ENGINE", "0"))
 for name in names:
     g = dict(np.load(os.path.join("tests/golden", name)))
     K = mo.tau_kernel(g["tau"], g["omega"], None)
     delta = mo.omega_delta(g["omega"]); D = mo.flat_default_model(g["omega"])
     t0 = time.time()
     prob = engine.SharedProblem(K, g["err"], D, delta, variant=str(g["variant"]),
-                                reduce_singular_space=float(g["reduce_singular_space"]), svd=svd, engine=engine_id)
+                                reduce_singular_space=float(g["reduce_singular_space"]), svd=svd)
     torch.cuda.synchronize(); t1 = time.time()
     res = engine.run_sweep(prob, g["G"], g["ref_alpha"], probability=bool(g["use_probability"]))
     torch.cuda.synchronize(); t2 = time.time()
