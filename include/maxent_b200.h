@@ -144,6 +144,11 @@ int mx_layout_V(const double* V, int32_t n_omega, int32_t n_sv, double* Vt, void
 int mx_tau_kernel(const double* tau, const double* omega, int32_t n_tau, int32_t n_omega,
                   double beta, double* K, void* stream);
 
+/* IOmegaKernel.fused_matrix (python/kernels.py:283-346): the stacked real kernel K[2 n_iw, n_omega] on the device,
+ * rows i < n_iw: Re 1/(i nu_i - omega) = -omega / (nu^2 + omega^2), rows n_iw + i: Im = -nu / (nu^2 + omega^2)
+ * (iomega = the real Matsubara frequencies nu_i). */
+int mx_iomega_kernel(const double* iomega, const double* omega, int32_t n_iw, int32_t n_omega, double* K, void* stream);
+
 /* One-sided (Hestenes) Jacobi SVD of K[m, n] (m >= n), every column: replaces np.linalg.svd in KernelSVD.svd
  * (python/kernels.py:53-64).  U[m, n], S[n] (descending), V[n, n]; work = m*n + n*n + n + 64 doubles.  One persistent
  * cooperative kernel, convergence decided on the device; `sweeps_done` (host, may be NULL) is filled by a
@@ -213,6 +218,20 @@ int mx_poorman_models(const double* A_out /*[R, MX_N_ANALYZERS, n_omega]*/, int3
                       int32_t P, const double* delta, double d_add, const double* A_init /*[n_omega] or NULL*/,
                       const double* Vp, const int32_t* group /*[P] or NULL*/, int32_t n_omega, int32_t n_sv,
                       double* D /*[P, ldD]*/, double* v0 /*[P, n_sv]*/, int32_t* ok /*[P]*/, void* stream);
+
+/* Retarded transform of spectra A(omega) that are linear between the omega nodes and zero outside them:
+ * G(z_k) = int dx A(x) / (z_k - x), z_k = w_k + i eta, eta > 0 (get_G_w_from_A_w, python/maxent_util.py, without the
+ * TRIQS containers).  Linear in A: G(z_k) = sum_j M[k, j] A_j.
+ * mx_hilbert_table builds M[n_w, n_omega] (complex, re/im interleaved; omega strictly increasing, n_omega >= 2).
+ * mx_hilbert_apply writes out[R, n_w] (complex, interleaved) for the rows A + r * lda (lda >= n_omega, r < R):
+ *   mode 0: G;  mode 1: scale[r] G + shift[r];  mode 2: z_k + shift[r] - 1/G
+ * (scale and shift [R], real, may be NULL: 1 and 0; w[n_w] is read in mode 2 only).  M and out 16-byte aligned.
+ * A row holding a NaN gives a NaN row.  The caller guarantees that the R rows of lda doubles lie inside A. */
+int mx_hilbert_table(const double* omega, int32_t n_omega, const double* w, int32_t n_w, double eta, double* M,
+                     void* stream);
+int mx_hilbert_apply(const double* A, int64_t lda, int32_t R, const double* M, int32_t n_omega, int32_t n_w,
+                     const double* w, double eta, int32_t mode, const double* scale, const double* shift, double* out,
+                     void* stream);
 
 #ifdef __cplusplus
 }

@@ -58,6 +58,7 @@ SYMBOLS = [
     ("mx_layout_V_size", ctypes.c_int64, [ctypes.c_int32, ctypes.c_int32]),
     ("mx_layout_V", ctypes.c_int, [c_dp, ctypes.c_int32, ctypes.c_int32, c_dp, c_dp]),
     ("mx_tau_kernel", ctypes.c_int, [c_dp, c_dp, ctypes.c_int32, ctypes.c_int32, ctypes.c_double, c_dp, c_dp]),
+    ("mx_iomega_kernel", ctypes.c_int, [c_dp, c_dp, ctypes.c_int32, ctypes.c_int32, c_dp, c_dp]),
     ("mx_svd_jacobi", ctypes.c_int, [c_dp, ctypes.c_int32, ctypes.c_int32, c_dp, c_dp, c_dp, c_dp,
                                      ctypes.c_int32, ctypes.POINTER(ctypes.c_int32), c_dp]),
     ("mx_gram_schmidt_rows", ctypes.c_int, [c_dp, ctypes.c_int32, ctypes.c_int32, ctypes.c_double, ctypes.c_void_p]),
@@ -73,6 +74,9 @@ SYMBOLS = [
                                   ctypes.c_double, ctypes.c_int32, ctypes.c_int32, c_dp, c_dp, c_dp, c_dp]),
     ("mx_poorman_models", ctypes.c_int, [c_dp, ctypes.c_int32, c_dp, ctypes.c_int32, c_dp, ctypes.c_double, c_dp, c_dp,
                                          c_dp, ctypes.c_int32, ctypes.c_int32, c_dp, c_dp, c_dp, c_dp]),
+    ("mx_hilbert_table", ctypes.c_int, [c_dp, ctypes.c_int32, c_dp, ctypes.c_int32, ctypes.c_double, c_dp, c_dp]),
+    ("mx_hilbert_apply", ctypes.c_int, [c_dp, ctypes.c_int64, ctypes.c_int32, c_dp, ctypes.c_int32, ctypes.c_int32, c_dp,
+                                        ctypes.c_double, ctypes.c_int32, c_dp, c_dp, c_dp, c_dp]),
 ]
 
 _lib = None

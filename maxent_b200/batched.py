@@ -121,6 +121,9 @@ class _BatchPlan(object):
 class BatchedTauMaxEnt(object):
     """MaxEnt continuation of a batch G[B, n_tau] sharing tau grid, omega mesh, error model and alpha mesh.
 
+    Matsubara data G(i omega_n)[B, n_iw] (``set_G_iw_data``) enter as the stacked real rows [Re G; Im G] of the
+    IOmegaKernel (python/kernels.py:283-346, ``kernels.IOmegaKernel.fused_matrix``); A(omega) stays real.
+
     Parameters mirror MaxEntLoop.__init__ (python/maxent_loop.py:83-94): ``cost_function`` in
     {'normal', 'plusminus', 'bryan'}, ``probability`` in {None, 'normal'}, ``reduce_singular_space``,
     ``scale_alpha`` ('Ndata' | number | None), ``G_threshold``."""
@@ -149,6 +152,7 @@ class BatchedTauMaxEnt(object):
         self.A_init = None
         self.tau = None
         self.beta = None
+        self.iomega = None                # Matsubara frequencies nu_n: the kernel is IOmegaKernel(iomega, omega)
         self.K = None                     # explicit kernel matrix (DataKernel) or None -> TauKernel(tau, omega, beta)
         self.err = None
         self.cov = None
@@ -166,12 +170,28 @@ class BatchedTauMaxEnt(object):
         if omega is not None:
             self.omega = omega if hasattr(omega, "delta") else DataOmegaMesh(omega)
         self.K = None
+        self.iomega = None
+        self.problem = None
+
+    def set_kernel_iw(self, iomega, omega=None):
+        """IOmegaKernel (python/kernels.py:283-346): K(i nu_n, omega) = 1 / (i nu_n - omega), ``iomega`` = the real
+        Matsubara frequencies nu_n.  The sweep sees the stacked real kernel [Re K; Im K] (2 n_iw rows)."""
+        iomega = np.array(iomega, dtype=np.float64).reshape(-1)
+        if len(iomega) < 1:
+            raise Exception("no Matsubara frequencies")
+        if self.cov is not None:
+            raise NotImplementedError("a covariance matrix of Matsubara data is not supported (IOmegaKernel.transform)")
+        self.iomega = iomega
+        if omega is not None:
+            self.omega = omega if hasattr(omega, "delta") else DataOmegaMesh(omega)
+        self.tau = self.beta = self.K = None
         self.problem = None
 
     def set_kernel_data(self, K, omega):
         """DataKernel (python/kernels.py:183-207): K[n_tau, n_omega] verbatim."""
         self.K = np.asarray(K, dtype=np.float64)
         self.omega = omega if hasattr(omega, "delta") else DataOmegaMesh(omega)
+        self.iomega = None
         self.problem = None
 
     def set_alpha_mesh_log(self, alpha_min, alpha_max, n_points):
@@ -180,10 +200,35 @@ class BatchedTauMaxEnt(object):
     def set_G_tau_data(self, tau, G):
         """tau[n_tau], G[B, n_tau] (python/tau_maxent.py:181-196, batched)."""
         G = np.asarray(G) if not hasattr(G, "data_ptr") else G
+        if G.is_complex() if hasattr(G, "is_complex") else np.iscomplexobj(G):
+            raise NotImplementedError("complex G(tau) is not continued by BatchedTauMaxEnt: Matsubara data go through "
+                                      "set_G_iw_data, complex matrix elements through BatchedElementwiseMaxEnt")
         if G.shape[-1] != len(tau):
             raise Exception("tau and G_tau don't have the same length")
         if self.tau is None or len(self.tau) != len(tau) or np.any(self.tau != np.asarray(tau)):
             self.set_kernel_tau(tau, None, None)
+        self.G = G
+
+    def set_G_iw_data(self, iomega, G_iw):
+        """iomega[n_iw] (real Matsubara frequencies), G_iw[B, n_iw] complex (numpy or tensor): kept as the stacked real
+        rows [Re G_iw, Im G_iw] of [B, 2 n_iw] that the IOmegaKernel's fused matrix continues."""
+        iomega = np.asarray(iomega, dtype=np.float64).reshape(-1)
+        if hasattr(G_iw, "data_ptr"):
+            import torch
+            G = G_iw if G_iw.dim() > 1 else G_iw[None, :]
+            if G.dim() != 2:
+                raise NotImplementedError("G_iw must be [B, n_iw]: matrix-valued Matsubara data are not supported")
+            G = torch.cat([G.real, G.imag] if G.is_complex() else [G, torch.zeros_like(G)], dim=1).to(torch.float64)
+        else:
+            G = np.asarray(G_iw)
+            G = G if G.ndim > 1 else G[None, :]
+            if G.ndim != 2:
+                raise NotImplementedError("G_iw must be [B, n_iw]: matrix-valued Matsubara data are not supported")
+            G = np.ascontiguousarray(np.concatenate([G.real, G.imag], axis=1), dtype=np.float64)
+        if G.shape[1] != 2 * len(iomega):
+            raise Exception("iomega and G_iw don't have the same length")
+        if self.iomega is None or len(self.iomega) != len(iomega) or np.any(self.iomega != iomega):
+            self.set_kernel_iw(iomega, None)
         self.G = G
 
     def set_error(self, err, per_spectrum=None):
@@ -212,6 +257,8 @@ class BatchedTauMaxEnt(object):
         """Covariance matrix of the data, [n_tau, n_tau] shared by the batch or [B, n_tau, n_tau] per spectrum
         (TauMaxEnt.set_cov, python/tau_maxent.py:253-288): rotate into the eigenbasis, errors = sqrt(eigenvalues),
         eigenvalues below ``cov_threshold`` dropped.  Identical matrices share one whitening group."""
+        if self.iomega is not None:
+            raise NotImplementedError("a covariance matrix of Matsubara data is not supported (IOmegaKernel.transform)")
         cov = np.asarray(cov, dtype=np.float64)
         assert np.max(np.abs(cov - np.swapaxes(cov, -1, -2))) < 1.e-10, 'Supplied covariance matrix is not symmetric.'
         self.cov = cov
@@ -226,7 +273,7 @@ class BatchedTauMaxEnt(object):
         ('groups', index[B], specs) with one spec = (T or None, error vector) per whitening group.  The groups of
         err[B, n_tau] are numbered in the sorted order of their vectors, those of cov[B, n, n] in the order of first
         appearance."""
-        n_tau = len(self.tau) if self.tau is not None else self.K.shape[0]
+        n_tau = self._n_rows()
         if self.cov is not None:
             covs = self.cov if self.cov.ndim == 3 else self.cov[None]
             if self.cov.ndim == 3 and covs.shape[0] != B:
@@ -245,12 +292,12 @@ class BatchedTauMaxEnt(object):
             return "groups", index, specs
         if self.err is None:
             raise Exception("no error set: call set_error")
-        err = np.asarray(self.err, dtype=np.float64)
+        err, per_spectrum = self._row_error()
         if self._groups is not None:
             if self._groups.shape != (B,) or err.ndim != 2 or err.shape[1] != n_tau:
                 raise Exception("error groups: %s vectors for %d spectra, index %s" % (err.shape, B, self._groups.shape))
             return "groups", self._groups, [(None, e) for e in err]
-        if err.ndim == 0 or (err.ndim == 1 and err.shape[0] == n_tau and not self._per_spectrum):
+        if err.ndim == 0 or (err.ndim == 1 and err.shape[0] == n_tau and not per_spectrum):
             return "shared", None, None
         if err.ndim == 1:
             if err.shape[0] != B:
@@ -279,15 +326,40 @@ class BatchedTauMaxEnt(object):
             plan.alpha = np.asarray(self.alpha_mesh, dtype=np.float64)
             plan.alpha_scale = np.array([rows[g] for g in index], dtype=np.float64)
         elif isinstance(self.scale_alpha, str):
-            plan.alpha = np.asarray(self.alpha_mesh, dtype=np.float64) * rows[0]
+            plan.alpha = np.asarray(self.alpha_mesh, dtype=np.float64) * self._n_data(rows[0])
         return plan
+
+    def _n_rows(self):
+        """Rows of the data the sweep sees: n_tau, or 2 n_iw stacked rows of Matsubara data."""
+        if self.iomega is not None:
+            return 2 * len(self.iomega)
+        return len(self.tau) if self.tau is not None else self.K.shape[0]
+
+    def _n_data(self, n_rows):
+        """The number of data points scale_alpha = 'Ndata' counts for n_rows rows: Matsubara data count their complex
+        points, len(G) of MaxEntLoop._scale (python/maxent_loop.py:216-220), not the stacked rows."""
+        return n_rows // 2 if self.iomega is not None else n_rows
+
+    def _row_error(self):
+        """(err, per_spectrum) in the rows the sweep sees: an error per Matsubara point ([n_iw] or [G, n_iw]) is repeated
+        for the Re and Im rows (IOmegaKernel.stack); for Matsubara data a 1-D error not of length n_iw is one per
+        spectrum."""
+        err = np.asarray(self.err, dtype=np.float64)
+        if self.iomega is None or err.ndim == 0:
+            return err, self._per_spectrum
+        n_iw = len(self.iomega)
+        if err.ndim == 1 and (self._per_spectrum or err.shape[0] != n_iw):
+            return err, True
+        if err.shape[-1] != n_iw:
+            raise Exception("error array has shape %s, the data have %d Matsubara points" % (err.shape, n_iw))
+        return np.concatenate([err, err], axis=-1), False
 
     # ---- run --------------------------------------------------------------------------------------
     def prepare(self):
         """Everything that depends on the kernel only (KernelSVD, truncation, layout); cached, and rebuilt when one of the
         public attributes it depends on was replaced (D, A_init, omega, reduce_singular_space, cost_function, svd)."""
         key = (self.cost_function, None if self.reduce_singular_space is None else float(self.reduce_singular_space), self.svd,
-               id(self.omega), id(self.D), id(self.A_init), id(self.K), id(self.tau), self.beta)
+               id(self.omega), id(self.D), id(self.A_init), id(self.K), id(self.tau), self.beta, id(self.iomega))
         if self.problem is not None and getattr(self, "_problem_key", None) == key:
             return self.problem
         self._problem_key = key
@@ -299,13 +371,20 @@ class BatchedTauMaxEnt(object):
         lib = _lib.load()
         omega = self.omega
         with torch.cuda.device(dev):
-            if self.K is None:
+            stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+            if self.iomega is not None:
+                i_d = torch.as_tensor(self.iomega, device=dev)
+                o_d = torch.as_tensor(np.asarray(omega, dtype=np.float64), device=dev)
+                K = torch.empty((2 * len(self.iomega), len(omega)), dtype=torch.float64, device=dev)
+                _lib.check(lib.mx_iomega_kernel(i_d.data_ptr(), o_d.data_ptr(), len(self.iomega), len(omega),
+                                                K.data_ptr(), stream), "mx_iomega_kernel")
+            elif self.K is None:
                 if self.tau is None:
-                    raise Exception("no kernel: call set_G_tau_data / set_kernel_tau / set_kernel_data first")
+                    raise Exception("no kernel: call set_G_tau_data / set_G_iw_data / set_kernel_tau / set_kernel_data "
+                                    "first")
                 t_d = torch.as_tensor(self.tau, device=dev)
                 o_d = torch.as_tensor(np.asarray(omega, dtype=np.float64), device=dev)
                 K = torch.empty((len(self.tau), len(omega)), dtype=torch.float64, device=dev)
-                stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
                 _lib.check(lib.mx_tau_kernel(t_d.data_ptr(), o_d.data_ptr(), len(self.tau), len(omega), self.beta,
                                              K.data_ptr(), stream), "mx_tau_kernel")
             else:
@@ -313,8 +392,8 @@ class BatchedTauMaxEnt(object):
         if self.err is None and self.cov is None:
             raise Exception("no error set: call set_error")
         D = FlatDefaultModel(omega).D if self.D is None else (self.D.D if hasattr(self.D, "D") else np.asarray(self.D))
-        err = np.asarray(1.0 if self.err is None else self.err, dtype=np.float64)
-        shared = err.ndim == 0 or (err.ndim == 1 and err.shape[0] == K.shape[0] and not self._per_spectrum)
+        err, per_spectrum = self._row_error() if self.err is not None else (np.float64(1.0), None)
+        shared = err.ndim == 0 or (err.ndim == 1 and err.shape[0] == K.shape[0] and not per_spectrum)
         # per-spectrum error models: the base problem carries err = 1 (kernel SVD, truncation, V layout); error scales
         # or whitening groups are attached per launch (run_device)
         self._K_dev, self._D_host = K, D
@@ -348,7 +427,7 @@ class BatchedTauMaxEnt(object):
         if isinstance(self.scale_alpha, str):
             if self.scale_alpha.lower() != "ndata":
                 raise Exception("Unknown value {} for scale_alpha".format(self.scale_alpha))
-            return a * self.prepare().n_tau
+            return a * self._n_data(self.prepare().n_tau)
         return a * float(self.scale_alpha)
 
     def run_device(self, G_dev, want_A=True, want_v=False, D=None, skip_small=False, v0=None):
@@ -357,14 +436,19 @@ class BatchedTauMaxEnt(object):
         ``v0`` [B, n_sv] the model rows are ready-made (D [B, ldD], engine.run_sweep).
         Per-spectrum error models (set_error / set_cov with a leading batch axis) are applied here.
         ``skip_small``: spectra with max|G| < G_threshold are NOT continued (python/maxent_loop.py:174-179): they are left
-        out of the launch and come back with status MX_STATUS_SKIPPED, NaN scalars, alpha_index -1 and A = 0."""
+        out of the launch and come back with status MX_STATUS_SKIPPED, NaN scalars, alpha_index -1 and A = 0.  For
+        Matsubara data (stacked rows [Re G; Im G]) |G| is the complex modulus, as MaxEntLoop.run takes it."""
         import torch
         skip = skip_small and G_dev.dim() > 1
         G = G_dev if G_dev.dim() > 1 else G_dev[None, :]
         B = int(G.shape[0])
         plan = self._batch_plan(B)
         if skip and B:
-            small = G.abs().amax(dim=1) < self.G_threshold
+            if self.iomega is not None:
+                n_iw = G.shape[1] // 2
+                small = torch.hypot(G[:, :n_iw], G[:, n_iw:]).amax(dim=1) < self.G_threshold
+            else:
+                small = G.abs().amax(dim=1) < self.G_threshold
             if bool(small.any()):
                 keep = torch.nonzero(~small).flatten()
                 kept = keep.cpu().numpy()
@@ -438,7 +522,9 @@ class BatchedTauMaxEnt(object):
         import torch
         G = self.G if G is None else G
         if G is None:
-            raise Exception("no data: call set_G_tau_data")
+            raise Exception("no data: call set_G_tau_data or set_G_iw_data")
+        if G.is_complex() if torch.is_tensor(G) else np.iscomplexobj(G):
+            raise NotImplementedError("complex data: pass G(i omega_n) through set_G_iw_data")
         prob = self.prepare()
         dev = prob.device
         Gt = G if torch.is_tensor(G) else torch.from_numpy(np.ascontiguousarray(G, dtype=np.float64))

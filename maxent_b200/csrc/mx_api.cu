@@ -1,5 +1,5 @@
 // C ABI of maxent_b200 (include/maxent_b200.h) + the small kernels around the alpha sweep:
-// V' re-tiling, TauKernel fill, data projection, analyzer reductions.
+// V' re-tiling, TauKernel and IOmegaKernel fills, data projection, analyzer reductions.
 #include <stdlib.h>
 #include "mx_common.cuh"
 #include <stdio.h>
@@ -35,6 +35,33 @@ __global__ void tau_kernel_kernel(const double* __restrict__ tau, const double* 
         if (w >= 0.0) v = -exp(-w * t) / (exp(-beta * w) + 1.0);
         else          v = -exp(w * (beta - t)) / (1.0 + exp(beta * w));
         K[o] = v;
+    }
+}
+
+// ---- IOmegaKernel.fused_matrix (python/kernels.py:283-346): K[2 n_iw, n_omega] = [Re; Im] 1 / (i nu_n - omega) ----
+// Evaluated as numpy divides complex numbers (Smith's algorithm on 1 / (-omega + i nu), no contracted products), so that
+// the device fill reproduces the host matrix of IOmegaKernel to the last bits.
+__global__ void iomega_kernel_kernel(const double* __restrict__ iomega, const double* __restrict__ omega,
+                                     int n_iw, int n_omega, double* __restrict__ K) {
+    const int64_t total = (int64_t)n_iw * n_omega;
+    for (int64_t o = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; o < total; o += (int64_t)gridDim.x * blockDim.x) {
+        const int i = (int)(o / n_omega), j = (int)(o - (int64_t)i * n_omega);
+        const double br = -omega[j], bi = iomega[i];         // denominator br + i bi
+        double re, im;
+        if (fabs(br) >= fabs(bi)) {
+            if (br == 0.0 && bi == 0.0) { re = 1.0 / fabs(br); im = 0.0 / fabs(br); }
+            else {
+                const double rat = bi / br, scl = 1.0 / __dadd_rn(br, __dmul_rn(bi, rat));
+                re = __dmul_rn(__dadd_rn(1.0, __dmul_rn(0.0, rat)), scl);
+                im = __dmul_rn(__dsub_rn(0.0, rat), scl);
+            }
+        } else {
+            const double rat = br / bi, scl = 1.0 / __dadd_rn(bi, __dmul_rn(br, rat));
+            re = __dmul_rn(__dadd_rn(rat, 0.0), scl);
+            im = __dmul_rn(__dsub_rn(__dmul_rn(0.0, rat), 1.0), scl);
+        }
+        K[o] = re;
+        K[o + total] = im;
     }
 }
 
@@ -333,6 +360,14 @@ int mx_tau_kernel(const double* tau, const double* omega, int32_t n_tau, int32_t
     const int64_t total = (int64_t)n_tau * n_omega;
     const int grid = (int)((total + 255) / 256 < 1184 ? (total + 255) / 256 : 1184);
     tau_kernel_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(tau, omega, n_tau, n_omega, beta, K);
+    return cudaGetLastError() == cudaSuccess ? MX_OK : MX_ERR_CUDA;
+}
+
+int mx_iomega_kernel(const double* iomega, const double* omega, int32_t n_iw, int32_t n_omega, double* K, void* stream) {
+    if (!iomega || !omega || !K || n_iw < 1 || n_omega < 1) return MX_ERR_BAD_ARG;
+    const int64_t total = (int64_t)n_iw * n_omega;
+    const int grid = (int)((total + 255) / 256 < 1184 ? (total + 255) / 256 : 1184);
+    iomega_kernel_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(iomega, omega, n_iw, n_omega, K);
     return cudaGetLastError() == cudaSuccess ? MX_OK : MX_ERR_CUDA;
 }
 

@@ -4,6 +4,8 @@
     torch.ops.maxent_b200.alpha_sweep     -> mx_alpha_sweep
     torch.ops.maxent_b200.analyze         -> mx_analyze
     torch.ops.maxent_b200.poorman_models  -> mx_poorman_models
+    torch.ops.maxent_b200.hilbert_table   -> mx_hilbert_table
+    torch.ops.maxent_b200.hilbert_apply   -> mx_hilbert_apply
 
 The operators are registered for the CUDA dispatch key ONLY: calling one with host tensors raises
 ``NotImplementedError`` from the dispatcher -- there is no CPU implementation of the hot path.  They are thin:
@@ -15,6 +17,7 @@ Reference seam these replace: the body of MaxEntLoop.run (python/maxent_loop.py:
 MaxEntResult.analyze (python/maxent_result.py:795-818).
 """
 import ctypes
+import math
 
 import torch
 
@@ -36,6 +39,9 @@ _library.define("analyze(Tensor alpha, Tensor chi2, Tensor S, Tensor? logp, Tens
                 "bool bryan_by_integration, Tensor(a!) alpha_index, Tensor(b!)? A_out, Tensor(c!)? aux) -> ()")
 _library.define("poorman_models(Tensor A_out, int slot, Tensor rows, Tensor delta, float d_add, Tensor? A_init, Tensor Vp, "
                 "Tensor? group, Tensor(a!) D, Tensor(b!) v0, Tensor(c!) ok) -> ()")
+_library.define("hilbert_table(Tensor omega, Tensor w, float eta, Tensor(a!) M) -> ()")
+_library.define("hilbert_apply(Tensor A, Tensor M, Tensor w, float eta, int mode, Tensor? scale, Tensor? shift, "
+                "Tensor(a!) out) -> ()")
 
 
 def _ptr(t):
@@ -134,13 +140,93 @@ def _poorman_models(A_out, slot, rows, delta, d_add, A_init, Vp, group, D, v0, o
                                                  _ptr(D), _ptr(v0), _ptr(ok), _stream(A_out)), "mx_poorman_models")
 
 
+def _vector(t, n, what):
+    if t.dtype != torch.float64 or not t.is_contiguous() or t.shape != (n,):
+        raise ValueError("%s must be a contiguous float64 tensor of shape (%d,)" % (what, n))
+
+
+def _eta(eta):
+    if not (math.isfinite(eta) and eta > 0.0):
+        raise ValueError("eta must be a finite number > 0, got %r" % (eta,))
+
+
+def check_hilbert_table(omega, w, eta, M):
+    """Every size mx_hilbert_table uses, checked before the launch: omega[n_omega >= 2], w[n_w] contiguous float64,
+    M complex128 [n_w, n_omega] contiguous, eta > 0.  Returns (n_omega, n_w).  (That omega increases strictly is the
+    caller's guarantee: real_frequency checks it on the host mesh.)"""
+    n_omega, n_w = int(omega.numel()), int(w.numel())
+    if n_omega < 2:
+        raise ValueError("the omega mesh needs at least two points")
+    _vector(omega, n_omega, "omega")
+    _vector(w, n_w, "w")
+    _eta(eta)
+    if M.dtype != torch.complex128 or not M.is_contiguous() or M.shape != (n_w, n_omega):
+        raise ValueError("M must be a contiguous complex128 tensor of shape (%d, %d)" % (n_w, n_omega))
+    if len({t.device for t in (omega, w, M)}) != 1:
+        raise ValueError("omega, w and M must be on one device")
+    return n_omega, n_w
+
+
+def check_hilbert_apply(A, M, w, eta, mode, scale, shift, out):
+    """Every index and size mx_hilbert_apply uses, checked before the launch.  A is [R, n_omega] float64 with unit column
+    stride and any row stride lda >= n_omega (e.g. A_out[:, slot] of an analyzer output [B, 5, n_omega], read in place);
+    torch keeps every view inside its storage.  M complex128 [n_w, n_omega], w float64 [n_w], scale and shift
+    float64 [R] or None, out complex128 [R, n_w], all contiguous and on A's device; mode 0 / 1 / 2, eta > 0.
+    Returns (lda, R, n_omega, n_w)."""
+    if A.dtype != torch.float64 or A.dim() != 2 or (A.shape[1] > 1 and A.stride(1) != 1):
+        raise ValueError("A must be a float64 matrix [R, n_omega] with contiguous rows")
+    R, n_omega = int(A.shape[0]), int(A.shape[1])
+    if n_omega < 1:
+        raise ValueError("A has no omega points")
+    lda = int(A.stride(0)) if R > 1 else max(int(A.stride(0)), n_omega)
+    if lda < n_omega:
+        raise ValueError("the rows of A overlap (row stride %d < n_omega %d)" % (lda, n_omega))
+    if M.dtype != torch.complex128 or not M.is_contiguous() or M.dim() != 2 or int(M.shape[1]) != n_omega:
+        raise ValueError("M must be a contiguous complex128 tensor [n_w, %d]" % n_omega)
+    n_w = int(M.shape[0])
+    if n_w < 1:
+        raise ValueError("M has no frequencies")
+    _vector(w, n_w, "w")
+    _eta(eta)
+    if int(mode) not in (0, 1, 2):
+        raise ValueError("mode must be 0 (G), 1 (scale G + shift) or 2 (z + shift - 1/G)")
+    for t, what in ((scale, "scale"), (shift, "shift")):
+        if t is not None:
+            _vector(t, R, what)
+    if out.dtype != torch.complex128 or not out.is_contiguous() or out.shape != (R, n_w):
+        raise ValueError("out must be a contiguous complex128 tensor of shape (%d, %d)" % (R, n_w))
+    if len({t.device for t in (A, M, w, scale, shift, out) if t is not None}) != 1:
+        raise ValueError("the tensors of hilbert_apply must be on one device")
+    return lda, R, n_omega, n_w
+
+
+def _hilbert_table(omega, w, eta, M):
+    n_omega, n_w = check_hilbert_table(omega, w, eta, M)
+    with torch.cuda.device(M.device):
+        _lib.check(_lib.load().mx_hilbert_table(_ptr(omega), n_omega, _ptr(w), n_w, float(eta), _ptr(M), _stream(M)),
+                   "mx_hilbert_table")
+
+
+def _hilbert_apply(A, M, w, eta, mode, scale, shift, out):
+    lda, R, n_omega, n_w = check_hilbert_apply(A, M, w, eta, mode, scale, shift, out)
+    if R == 0:
+        return
+    with torch.cuda.device(out.device):
+        _lib.check(_lib.load().mx_hilbert_apply(_ptr(A), lda, R, _ptr(M), n_omega, n_w, _ptr(w), float(eta), int(mode),
+                                                _ptr(scale), _ptr(shift), _ptr(out), _stream(out)), "mx_hilbert_apply")
+
+
 _library.impl("project_data", _project_data, "CUDA")
 _library.impl("alpha_sweep", _alpha_sweep, "CUDA")
 _library.impl("analyze", _analyze, "CUDA")
 _library.impl("poorman_models", _poorman_models, "CUDA")
+_library.impl("hilbert_table", _hilbert_table, "CUDA")
+_library.impl("hilbert_apply", _hilbert_apply, "CUDA")
 
 project_data = torch.ops.maxent_b200.project_data
 alpha_sweep = torch.ops.maxent_b200.alpha_sweep
 analyze = torch.ops.maxent_b200.analyze
 poorman_models = torch.ops.maxent_b200.poorman_models
-OPERATORS = ("project_data", "alpha_sweep", "analyze", "poorman_models")
+hilbert_table = torch.ops.maxent_b200.hilbert_table
+hilbert_apply = torch.ops.maxent_b200.hilbert_apply
+OPERATORS = ("project_data", "alpha_sweep", "analyze", "poorman_models", "hilbert_table", "hilbert_apply")
