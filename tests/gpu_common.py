@@ -64,6 +64,31 @@ def run_fixture(g, svd="jacobi", B=1, **kw):
     return prob, res
 
 
+def sweep_tiles(n_sv):
+    """Tile count NT of the sweep instantiation for n_sv (sweep_tiles in mx_common.cuh): 8 columns per tile, at least
+    4, multiples of 4 above 10 (the wide instantiations)."""
+    nt = max((n_sv + 7) // 8, 4)
+    return (nt + 3) & ~3 if nt > 10 else nt
+
+
+def kernel_problem(n_sv, n_tau, n_om, variant, seed, n_spectra):
+    """A DataKernel K = U diag(logspace(0, -6, n_sv)) V^T plus a floor of 1e-14, with exactly n_sv singular values above
+    the cut 1e-9 (the construction of test_gpu_parity; n_tau >= n_om), and n_spectra noisy data sets of a two-peak
+    spectrum (plus-minus: with a negative lobe).  Returns (K, G, omega, delta)."""
+    rng = np.random.RandomState(seed)
+    om = mo.linear_omega_mesh(-4, 4, n_om)
+    U, _ = np.linalg.qr(rng.randn(n_tau, n_om))
+    V, _ = np.linalg.qr(rng.randn(n_om, n_om))
+    S = np.concatenate([np.logspace(0, -6, n_sv), 1e-14 * np.ones(n_om - n_sv)])
+    K = (U * S) @ V.T
+    A_true = np.exp(-(om - 0.5) ** 2) + 0.5 * np.exp(-(om + 1.5) ** 2 / 0.5)
+    if variant == "plusminus":
+        A_true = A_true - 0.8 * np.exp(-(om - 2.0) ** 2 / 0.3)
+    delta = mo.omega_delta(om)
+    G = (K * delta[None, :]) @ A_true + 1e-4 * rng.randn(n_spectra, n_tau)
+    return K, G, om, delta
+
+
 def rel_A(A, Aref):
     return np.max(np.abs(A - Aref), axis=-1) / np.max(np.abs(Aref), axis=-1)
 

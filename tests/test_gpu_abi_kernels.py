@@ -92,11 +92,6 @@ def _tile_off(n, c):
     return 16 * q + 2 * ((4 * e + cc + 2 * q) & 7) + h
 
 
-def _sweep_tiles(n_sv):
-    nt = max((n_sv + 7) // 8, 4)
-    return (nt + 3) & ~3 if nt > 10 else nt
-
-
 @pytest.mark.parametrize("n_sv", [1, 7, 8, 9, 52, 80, 81, 96, 200, 256])
 def test_layout_V_inverts_tile_off(torch_cuda, lib, n_sv):
     """V'[n_omega, n_sv] -> [n_kt][NT][64] tiles: every element where the host inverse of tile_off puts it, exact zeros
@@ -110,7 +105,7 @@ def test_layout_V_inverts_tile_off(torch_cuda, lib, n_sv):
     rng = np.random.RandomState(n_sv)
     for n_omega in (1, 7, 8, 1001):
         V = rng.randn(n_omega, n_sv) + 3.0                             # no zeros: a zero in Vt is padding
-        NT, n_kt = _sweep_tiles(n_sv), (n_omega + 7) // 8
+        NT, n_kt = gc.sweep_tiles(n_sv), (n_omega + 7) // 8
         total = int(lib.mx_layout_V_size(n_omega, n_sv))
         assert total == n_kt * NT * 64
         Vt = torch.full((total,), float("nan"), dtype=torch.float64, device="cuda")
@@ -559,28 +554,12 @@ def test_poorman_models_position_independence(torch_cuda):
 # ----------------------------------------------------------------------------------------------
 # one sweep over whitening groups of different n_sv
 # ----------------------------------------------------------------------------------------------
-def _kernel_problem(n_sv, n_tau, n_om, variant, seed, n_spectra):
-    """A DataKernel with exactly n_sv singular values above the cut 1e-9 (the construction of test_gpu_parity)."""
-    rng = np.random.RandomState(seed)
-    om = mo.linear_omega_mesh(-4, 4, n_om)
-    U, _ = np.linalg.qr(rng.randn(n_tau, n_om))
-    V, _ = np.linalg.qr(rng.randn(n_om, n_om))
-    S = np.concatenate([np.logspace(0, -6, n_sv), 1e-14 * np.ones(n_om - n_sv)])
-    K = (U * S) @ V.T
-    A_true = np.exp(-(om - 0.5) ** 2) + 0.5 * np.exp(-(om + 1.5) ** 2 / 0.5)
-    if variant == "plusminus":
-        A_true = A_true - 0.8 * np.exp(-(om - 2.0) ** 2 / 0.3)
-    delta = mo.omega_delta(om)
-    G = (K * delta[None, :]) @ A_true + 1e-4 * rng.randn(n_spectra, n_tau)
-    return K, G, om, delta
-
-
 def _groups_run(variant, marquardt, n_svs, n_tau, n_om, n_alpha):
     from maxent_b200 import engine
     mesh = mo.log_alpha_mesh(0.5, 500, n_alpha)
     probs, Gs, Ks = [], [], []
     for g, s in enumerate(n_svs):
-        K, G, om, delta = _kernel_problem(s, n_tau, n_om, variant, 40 + g, 2)
+        K, G, om, delta = gc.kernel_problem(s, n_tau, n_om, variant, 40 + g, 2)
         q = engine.SharedProblem(K, 1e-4, mo.flat_default_model(om), delta, variant=variant, reduce_singular_space=1e-9)
         assert q.n_sv == s
         probs.append(q)
