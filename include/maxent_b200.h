@@ -25,6 +25,7 @@ extern "C" {
 #define MX_ERR_CUDA         -3
 #define MX_ERR_NO_DEVICE    -4
 
+#define MX_MAX_MATRIX        8   /* largest block size M of mx_matrix_resolvent */
 #define MX_MAX_NSV         256   /* singular-space dimension the fused path supports: up to 80 with every matrix in
                                     * shared memory and registers, 81..256 with Z, J and the factors in the workspace */
 
@@ -232,6 +233,19 @@ int mx_hilbert_table(const double* omega, int32_t n_omega, const double* w, int3
 int mx_hilbert_apply(const double* A, int64_t lda, int32_t R, const double* M, int32_t n_omega, int32_t n_w,
                      const double* w, double eta, int32_t mode, const double* scale, const double* shift, double* out,
                      void* stream);
+
+/* Batched shifted matrix inversion, the two matrix steps of the inversion method for matrix-valued self-energies
+ * (InversionSigmaContinuator, python/sigma_continuator.py, per matrix).  For every matrix b < B and frequency k < n_z,
+ * with X(b,k) = X[b, :, :, k] (complex, re/im interleaved, layout [B, M, M, n_z], frequency innermost), z[n_z] complex
+ * and C[B] real (NULL: 0):
+ *   mode 0: Y(b,k) = ((z_k + C_b) 1 - X(b,k))^{-1}        (G_aux from Sigma on the Matsubara axis)
+ *   mode 1: Y(b,k) = (z_k + C_b) 1 - X(b,k)^{-1}          (Sigma from G_aux(w + i eta))
+ * FP64 Gauss-Jordan with partial pivoting by modulus, in a fixed operation order: Y(b,k) does not depend on the rest of
+ * the batch.  Y has X's layout and may equal X.  A non-finite entry of X(b,k), or an exactly zero pivot, makes all of
+ * Y(b,k) NaN.  X, Y and z 16-byte aligned.  1 <= M <= MX_MAX_MATRIX, else MX_ERR_UNSUPPORTED; B == 0 or n_z == 0:
+ * MX_OK, no launch. */
+int mx_matrix_resolvent(const double* X, int32_t B, int32_t M, int32_t n_z, const double* z, const double* C,
+                        int32_t mode, double* Y, void* stream);
 
 #ifdef __cplusplus
 }

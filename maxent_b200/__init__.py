@@ -30,7 +30,7 @@ from .tau_maxent import TauMaxEnt
 from .elementwise_maxent import ElementwiseMaxEnt, DiagonalMaxEnt, PoormanMaxEnt, CallableMethodCheck
 from .batched import BatchedTauMaxEnt, BatchedMaxEntResult
 from .batched_matrix import BatchedElementwiseMaxEnt, BatchedPoormanMaxEnt, BatchedMatrixMaxEntResult
-from .real_frequency import BatchedSigmaContinuator, retarded_G
+from .real_frequency import BatchedSigmaContinuator, retarded_G, matrix_sigma_w
 from .maxent_util import numder, check_der, get_G_w_from_A_w, get_G_tau_from_A_w
 from .triqs_support import if_no_triqs, if_triqs_1, if_triqs_2, require_triqs, assert_text_files_equal
 from .version import show_version, show_git_hash

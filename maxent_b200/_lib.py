@@ -12,6 +12,7 @@ LIB_PATH = os.environ.get("MAXENT_B200_LIB") or os.path.join(HERE, "libmaxent_b2
 
 MX_OK = 0
 MX_MAX_NSV = 256
+MX_MAX_MATRIX = 8
 VARIANTS = {"normal": 0, "plusminus": 1, "bryan": 2}
 AN_LINEFIT, AN_CHI2CURV, AN_ENTROPY, AN_CLASSIC, AN_BRYAN = range(5)
 N_ANALYZERS = 5
@@ -77,6 +78,8 @@ SYMBOLS = [
     ("mx_hilbert_table", ctypes.c_int, [c_dp, ctypes.c_int32, c_dp, ctypes.c_int32, ctypes.c_double, c_dp, c_dp]),
     ("mx_hilbert_apply", ctypes.c_int, [c_dp, ctypes.c_int64, ctypes.c_int32, c_dp, ctypes.c_int32, ctypes.c_int32, c_dp,
                                         ctypes.c_double, ctypes.c_int32, c_dp, c_dp, c_dp, c_dp]),
+    ("mx_matrix_resolvent", ctypes.c_int, [c_dp, ctypes.c_int32, ctypes.c_int32, ctypes.c_int32, c_dp, c_dp, ctypes.c_int32,
+                                           c_dp, c_dp]),
 ]
 
 _lib = None

@@ -13,7 +13,11 @@ is the one of SURVEY.md 8(e):
    for Poorman).  With ``use_hermiticity`` only i < j is continued.
 
 Every spectrum is continued by its own CTA and the default models are summed in a fixed order, so a matrix's results do
-not depend on which other matrices share the batch."""
+not depend on which other matrices share the batch.
+
+Matsubara data G(i omega_n)[B, M, M, n_iw] (``set_G_iw_data``) go through the same schedule on the IOmegaKernel: every
+planned element (b, i, j, c) is continued as the stacked real rows [Re d; Im d] of ``matsubara_rows``, the exact Matsubara
+image of what the tau path continues (Re G_ij(tau) for c = 0, Im G_ij(tau) for c = 1)."""
 import numpy as np
 
 from . import _lib
@@ -31,6 +35,26 @@ def element_plan(B, M, use_hermiticity=True, use_complex=False):
     off = np.array([(b, i, j, c) for b in range(B) for i in range(M) for j in range(M)
                     if i != j and not (use_hermiticity and i > j) for c in parts], dtype=np.int64).reshape(-1, 4)
     return diag, off
+
+
+def matsubara_rows(G_iw, plan):
+    """Stacked real rows [Re d; Im d] [P, 2 n_iw] (float64, on G_iw's device) of the planned elements (b, i, j, c) of the
+    complex Matsubara data G_iw[B, M, M, n_iw] (tensor, any device):
+
+        c = 0:  d = (G_ij + G_ji) / 2        = K A'    (the transform of Re G_ij(tau))
+        c = 1:  d = (G_ij - G_ji) / (2i)     = K A''   (the transform of Im G_ij(tau))
+
+    for a Hermitian A = A' + i A'' and K = 1 / (i nu - omega).  The kernel is complex, so it mixes A' and A'': G_ij alone
+    does not separate them, and both G_ij and G_ji are read for every element.  Written with real operations only, so
+    that both are exact up to the one rounding of each sum; on the diagonal (x + x) / 2 == x, i.e. the rows of G_ii."""
+    import torch
+    Gr = torch.view_as_real(G_iw.to(torch.complex128))
+    idx = [torch.as_tensor(np.asarray(plan)[:, k], device=Gr.device) for k in range(4)]
+    gij, gji = Gr[idx[0], idx[1], idx[2]], Gr[idx[0], idx[2], idx[1]]          # [P, n_iw, 2]
+    sym = (gij + gji) / 2                                                     # c = 0: Re d, Im d
+    anti = torch.stack([gij[..., 1] - gji[..., 1], gji[..., 0] - gij[..., 0]], dim=-1) / 2     # c = 1
+    d = torch.where((idx[3] == 0)[:, None, None], sym, anti)
+    return torch.cat([d[..., 0], d[..., 1]], dim=1).contiguous()
 
 
 def synthetic_matrix_batch(n_tau, n_omega, B, seed=7, beta=40.0, sigma=1.e-4):
@@ -74,7 +98,8 @@ class BatchedMatrixMaxEntResult(object):
     A_out of (j, i) is taken from (i, j), imaginary part negated, as MaxEntResult.get_A_out does.  ``zero_elements[b]``
     lists the elements skipped below G_threshold (A = 0), ``skipped_elements[b]`` the Poorman off-diagonals whose
     diagonal partner had no A_out for ``analyzer_offdiag_D`` (A = NaN).  The full A_alpha(omega) stays on the device and
-    is copied on demand by ``A(b)``; ``result(b)`` (or ``out[b]``) is the MaxEntResult of matrix b."""
+    is copied on demand by ``A(b)``; ``result(b)`` (or ``out[b]``) is the MaxEntResult of matrix b.  For Matsubara data
+    its ``data_variable`` is ``iomega`` and G, G_rec are the stacked rows [Re; Im] that were continued."""
 
     def __len__(self):
         return int(self.chi2.shape[0])
@@ -112,6 +137,24 @@ class BatchedMatrixMaxEntResult(object):
                             A[i, j, 1] = -A[i, j, 1]
         return A
 
+    def A_out_device(self, slot):
+        """The analyzer slot of ``A_out`` assembled on the device from the two passes' analyzer output, without a trip to
+        the host: float64 [B, M, M, (2,) n_omega] (real and imaginary part on their own axis with complex elements), equal
+        bit for bit to A_out[..., slot, :] (zero below G_threshold, hermiticity copies with the imaginary part negated,
+        NaN for elements not continued or without a pick) with one exception: with ``use_hermiticity`` the transposed
+        element of one below G_threshold is zero here, where A_out keeps NaN (MaxEntResult.get_A_out lists the
+        continued element only), so that a matrix with an element below threshold still has a finite A_aux."""
+        import torch
+        parts = [res.A_out[:, slot] for res in self._device if res is not None]
+        dev, n_omega = parts[0].device, int(parts[0].shape[1])
+        special = torch.tensor([[float("nan")], [0.0]], dtype=torch.float64, device=dev).expand(2, n_omega)
+        table = torch.cat(parts + [special])
+        R = int(table.shape[0])
+        index = np.where(self._A_src == -1, R - 2, np.where(self._A_src == -2, R - 1, self._A_src))
+        A = table[torch.as_tensor(index.reshape(-1), device=dev)]
+        A = A * torch.as_tensor(self._A_sign.reshape(-1, 1), device=dev)
+        return A.reshape(self._A_src.shape + (n_omega,))
+
     def _key(self, i, j, c):
         return (i, j, c) if self.complex_elements else (i, j)
 
@@ -140,7 +183,8 @@ class BatchedMatrixMaxEntResult(object):
             key = self._key(i, j, c)
             record = dict(alpha=self.alpha, v=v, chi2=self.chi2[b][key], S=self.S[b][key], Q=self.Q[b][key],
                           A=A.cpu().numpy(), H=(A * prob.delta).cpu().numpy(), probability=self.probability[b][key],
-                          omega=self.omega, G=self._G_rows[k][r], G_orig=self._G_rows[k][r], data_variable=self.tau,
+                          omega=self.omega, G=self._G_rows[k][r], G_orig=self._G_rows[k][r],
+                          data_variable=self.tau if self.iomega is None else self.iomega,
                           G_rec=(A @ Kd.transpose(0, 1)).cpu().numpy(), n_iter=self.n_iter[b][key],
                           converged=self.converged[b][key], n_sv=prob.n_sv)
             out.add_sweep(record, matrix_element=(i, j), complex_index=c)
@@ -150,7 +194,8 @@ class BatchedMatrixMaxEntResult(object):
 
 class BatchedElementwiseMaxEnt(object):
     """ElementwiseMaxEnt (python/elementwise_maxent.py) for a batch of matrices G[B, M, M, n_tau] sharing tau grid,
-    omega mesh, alpha mesh and kernel: the off-diagonal elements use the off-diagonal worker's own default model."""
+    omega mesh, alpha mesh and kernel: the off-diagonal elements use the off-diagonal worker's own default model.
+    Matsubara matrices G[B, M, M, n_iw] enter through ``set_G_iw_data``."""
 
     def __init__(self, use_hermiticity=True, use_complex=False, probability=None, reduce_singular_space=1.e-14,
                  scale_alpha="Ndata", G_threshold=1.e-10, device=None, minimizer=None):
@@ -163,6 +208,7 @@ class BatchedElementwiseMaxEnt(object):
         self.probability = probability
         self.G = None
         self.tau = None
+        self.iomega = None
         self.error = None
         self.error_dimension = 1
 
@@ -199,7 +245,26 @@ class BatchedElementwiseMaxEnt(object):
             w.set_G_tau_data(tau, np.zeros((1, len(tau))))
             w.G = None
         self.tau = np.asarray(tau, dtype=np.float64)
+        self.iomega = None
         self.G = G
+
+    def set_G_iw_data(self, iomega, G_iw):
+        """iomega[n_iw] (real Matsubara frequencies), G_iw[B, M, M, n_iw] complex (numpy or torch): every planned element
+        is continued on the IOmegaKernel as the stacked rows of ``matsubara_rows``, which read G_ij and G_ji (also with
+        ``use_hermiticity``).  Error models as for tau data, with n_iw in place of n_tau; covariances are not supported."""
+        iomega = np.asarray(iomega, dtype=np.float64).reshape(-1)
+        if G_iw.ndim != 4 or G_iw.shape[1] != G_iw.shape[2]:
+            raise ValueError("G_iw must be [B, M, M, n_iw], got shape %s" % (tuple(G_iw.shape),))
+        if G_iw.shape[-1] != len(iomega):
+            raise Exception("iomega and G_iw don't have the same length")
+        if self.error_dimension == 2:
+            raise NotImplementedError("a covariance matrix of Matsubara data is not supported (IOmegaKernel.transform)")
+        for w in self._workers():
+            w.set_kernel_iw(iomega)
+            w.G = None
+        self.tau = None
+        self.iomega = iomega
+        self.G = G_iw
 
     def set_error(self, error, per_spectrum=None):
         """A scalar or a vector [n_tau] for every element; an array [M, M, n_tau] with one error vector per element
@@ -208,7 +273,10 @@ class BatchedElementwiseMaxEnt(object):
         self.error, self.error_dimension, self._per_spectrum = error, 1, per_spectrum
 
     def set_cov(self, cov):
-        """Covariance [n_tau, n_tau] shared by every element.  Per-element covariances are not supported."""
+        """Covariance [n_tau, n_tau] shared by every element.  Per-element covariances, and covariances of Matsubara data,
+        are not supported."""
+        if self.iomega is not None:
+            raise NotImplementedError("a covariance matrix of Matsubara data is not supported (IOmegaKernel.transform)")
         cov = np.asarray(cov, dtype=np.float64)
         if cov.ndim != 2:
             raise NotImplementedError("per-element covariance matrices [M, N, n_tau, n_tau] are not supported by the "
@@ -216,12 +284,14 @@ class BatchedElementwiseMaxEnt(object):
         self.error, self.error_dimension = cov, 2
 
     def _error_kind(self, B, M):
-        """'shared' | 'element' | 'spectrum' | 'cov' for the error set by set_error / set_cov (validates the shape)."""
+        """'shared' | 'element' | 'spectrum' | 'cov' for the error set by set_error / set_cov (validates the shape).  The
+        error counts data points: n_tau, or n_iw complex points of Matsubara data (the workers repeat a per-point error
+        for the Re and Im rows)."""
         if self.error is None:
             raise Exception("no error set: call set_error or set_cov")
         if self.error_dimension == 2:
             return "cov"
-        n_tau = len(self.tau)
+        n_tau = len(self.tau) if self.iomega is None else len(self.iomega)
         e = np.asarray(self.error, dtype=np.float64)
         if e.ndim == 0 or e.shape == (n_tau,):
             return "shared"
@@ -229,8 +299,9 @@ class BatchedElementwiseMaxEnt(object):
             return "element"
         if e.shape == (B, M, M):
             return "spectrum"
-        raise ValueError("error of shape %s: expected a scalar, [n_tau] = [%d], [M, M, n_tau] = %s or [B, M, M] = %s"
-                         % (e.shape, n_tau, (M, M, n_tau), (B, M, M)))
+        what = "n_tau" if self.iomega is None else "n_iw"
+        raise ValueError("error of shape %s: expected a scalar, [%s] = [%d], [M, M, %s] = %s or [B, M, M] = %s"
+                         % (e.shape, what, n_tau, what, (M, M, n_tau), (B, M, M)))
 
     def _put_error(self, worker, kind, plan):
         """Error model of the spectra `plan` (rows (b, i, j, c)) on `worker` (unchanged inputs keep the worker's
@@ -258,6 +329,8 @@ class BatchedElementwiseMaxEnt(object):
         dev = self.maxent_diagonal.prepare().device
         G = self.G if torch.is_tensor(self.G) else torch.from_numpy(np.ascontiguousarray(self.G))
         G = G.to(dev, non_blocking=True)
+        if self.iomega is not None:
+            return G.to(torch.complex128)
         if not G.is_complex():
             G = G.to(torch.float64)
             return torch.stack([G, torch.zeros_like(G)], dim=-1)
@@ -273,9 +346,13 @@ class BatchedElementwiseMaxEnt(object):
     def set_preblur(self, *args, **kwargs):
         raise NotImplementedError("preblur is not supported by the batched matrix path; use ElementwiseMaxEnt per matrix")
 
+    def _rows(self, Gd, plan):
+        """The device rows of the planned spectra: G(tau) rows, or the stacked Matsubara rows of ``matsubara_rows``."""
+        return self._gather(Gd, plan) if self.iomega is None else matsubara_rows(Gd, plan)
+
     def _check(self):
         if self.G is None:
-            raise Exception("no data: call set_G_tau_data")
+            raise Exception("no data: call set_G_tau_data or set_G_iw_data")
 
     def _offdiagonal_models(self, diag_res, off_plan, G2):
         """Default models of the off-diagonal pass: (G2, D, v0, not_ok) -- the worker's own model here."""
@@ -311,13 +388,13 @@ class BatchedElementwiseMaxEnt(object):
                 timeline.append(ev)
         with torch.cuda.device(dev):
             Gri = self._G_device()
-            G1 = self._gather(Gri, diag_plan)
+            G1 = self._rows(Gri, diag_plan)
             mark()
             r1 = self.maxent_diagonal.run_device(G1, want_A=True, want_v=True, skip_small=True)
             mark()
             if len(off_plan) == 0:
                 return (diag_plan, off_plan), (r1, None), (G1, None), None
-            G2 = self._gather(Gri, off_plan)
+            G2 = self._rows(Gri, off_plan)
             mark()
             G2, D, v0, not_ok = self._offdiagonal_models(r1, off_plan, G2)
             mark()
@@ -333,7 +410,7 @@ class BatchedElementwiseMaxEnt(object):
         out.matrix_structure = (M, M)
         out.use_hermiticity, out.complex_elements = self.use_hermiticity, self.use_complex
         out.probability_on = self.probability is not None
-        out.omega, out.tau = self.omega, self.tau
+        out.omega, out.tau, out.iomega = self.omega, self.tau, self.iomega
         out.alpha = self.maxent_diagonal.alpha_effective()
         out._plans, out._device = plans, results
         out._workers = self._workers()
@@ -365,6 +442,11 @@ class BatchedElementwiseMaxEnt(object):
         out.alpha_index = np.full(shp + (N_AN,), -1, dtype=np.int32)
         A_out = np.full(shp + (N_AN, n_omega), np.nan)
         computed = np.zeros(shp, dtype=bool)
+        # the source of every element's A_out, for the device assembly (A_out_device): row of the passes' analyzer output
+        # stacked in pass order, -1 NaN, -2 zero; times the sign of a hermiticity copy
+        src = np.full(shp, -1, dtype=np.int64)
+        sign = np.ones(shp)
+        first = np.cumsum([0] + [len(p) for p in plans])
         out.zero_elements = [[] for _ in range(B)]
         out.skipped_elements = [[] for _ in range(B)]
         zeros = []
@@ -389,6 +471,7 @@ class BatchedElementwiseMaxEnt(object):
                 out.alpha_index[key] = got["alpha_index"][r]
                 A_out[key] = got["A_out"][r]
                 computed[key] = True
+                src[key] = first[k] + r
             if k == 0 and self.use_complex:                      # a Hermitian matrix has a real diagonal
                 for b in range(B):
                     for i in range(M):
@@ -398,11 +481,21 @@ class BatchedElementwiseMaxEnt(object):
         # part that was not computed is taken from the computed transposed part, imaginary part negated
         for key in zeros:
             A_out[key] = np.where(np.asarray(computed[key])[..., None, None], A_out[key], 0.0)
+            src[key] = np.where(computed[key], src[key], -2)
         if self.use_hermiticity:
             A4, C4 = (A_out, computed) if self.use_complex else (A_out[:, :, :, None], computed[..., None])
+            S4, G4 = (src, sign) if self.use_complex else (src[..., None], sign[..., None])
             for b, i, j, c in zip(*np.nonzero(~C4)):
                 if i != j and C4[b, j, i, c]:
                     A4[b, i, j, c] = (-1.0 if self.use_complex and c == 1 else 1.0) * A4[b, j, i, c]
+                    S4[b, i, j, c] = S4[b, j, i, c]
+                    G4[b, i, j, c] = -1.0 if self.use_complex and c == 1 else 1.0
+            # the hermiticity image of an element below G_threshold is zero: NaN in A_out (only the listed element is
+            # zero there, as in MaxEntResult.get_A_out), zero in the device assembly that Sigma(w) is built from
+            for b, i, j, c in zip(*np.nonzero(S4 == -1)):
+                if i != j and S4[b, j, i, c] == -2:
+                    S4[b, i, j, c] = -2
+        out._A_src, out._A_sign = src, sign
         out.A_out = A_out[..., 0, :, :] + 1j * A_out[..., 1, :, :] if self.use_complex else A_out
 
 

@@ -21,7 +21,7 @@ SWEEP2_NT = (4, 5, 6, 7, 8, 9, 10, 12, 16, 20, 24, 28, 32)    # spectrum-per-CTA
 
 def _units():
     units = [("mx_api.o", "mx_api.cu", []), ("mx_svd.o", "mx_svd.cu", []), ("mx_dispatch.o", "mx_dispatch.cu", []),
-             ("mx_hilbert.o", "mx_hilbert.cu", [])]
+             ("mx_hilbert.o", "mx_hilbert.cu", []), ("mx_resolvent.o", "mx_resolvent.cu", [])]
     for nt in SWEEP2_NT:
         units.append(("mx_sweep2_nt%d.o" % nt, "mx_sweep2_inst.cu", ["-DMX_NT=%d" % nt]))
     return units

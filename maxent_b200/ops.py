@@ -6,6 +6,7 @@
     torch.ops.maxent_b200.poorman_models  -> mx_poorman_models
     torch.ops.maxent_b200.hilbert_table   -> mx_hilbert_table
     torch.ops.maxent_b200.hilbert_apply   -> mx_hilbert_apply
+    torch.ops.maxent_b200.matrix_resolvent -> mx_matrix_resolvent
 
 The operators are registered for the CUDA dispatch key ONLY: calling one with host tensors raises
 ``NotImplementedError`` from the dispatcher -- there is no CPU implementation of the hot path.  They are thin:
@@ -42,6 +43,7 @@ _library.define("poorman_models(Tensor A_out, int slot, Tensor rows, Tensor delt
 _library.define("hilbert_table(Tensor omega, Tensor w, float eta, Tensor(a!) M) -> ()")
 _library.define("hilbert_apply(Tensor A, Tensor M, Tensor w, float eta, int mode, Tensor? scale, Tensor? shift, "
                 "Tensor(a!) out) -> ()")
+_library.define("matrix_resolvent(Tensor X, Tensor z, Tensor? C, int mode, Tensor(a!) Y) -> ()")
 
 
 def _ptr(t):
@@ -216,12 +218,50 @@ def _hilbert_apply(A, M, w, eta, mode, scale, shift, out):
                                                 _ptr(scale), _ptr(shift), _ptr(out), _stream(out)), "mx_hilbert_apply")
 
 
+def check_matrix_resolvent(X, z, C, mode, Y):
+    """Every size mx_matrix_resolvent uses, checked before the launch: X complex128 [B, M, M, n_z] contiguous with
+    1 <= M <= MX_MAX_MATRIX, z complex128 [n_z] contiguous, C float64 [B] contiguous or None, Y like X (Y may be X itself,
+    but may not overlap it otherwise), all on one device; mode 0 ((z + C) 1 - X)^-1 or 1 (z + C) 1 - X^-1.
+    Returns (B, M, n_z)."""
+    if X.dtype != torch.complex128 or X.dim() != 4 or not X.is_contiguous():
+        raise ValueError("X must be a contiguous complex128 tensor [B, M, M, n_z]")
+    B, M, n_z = int(X.shape[0]), int(X.shape[1]), int(X.shape[3])
+    if int(X.shape[2]) != M:
+        raise ValueError("X must hold square matrices [B, M, M, n_z], got %s" % (tuple(X.shape),))
+    if not 1 <= M <= _lib.MX_MAX_MATRIX:
+        raise ValueError("the matrices must be M x M with 1 <= M <= %d, got M = %d" % (_lib.MX_MAX_MATRIX, M))
+    if z.dtype != torch.complex128 or not z.is_contiguous() or z.shape != (n_z,):
+        raise ValueError("z must be a contiguous complex128 tensor of shape (%d,)" % n_z)
+    if C is not None:
+        _vector(C, B, "C")
+    if int(mode) not in (0, 1):
+        raise ValueError("mode must be 0 (((z + C) 1 - X)^-1) or 1 ((z + C) 1 - X^-1)")
+    if Y.dtype != torch.complex128 or not Y.is_contiguous() or Y.shape != X.shape:
+        raise ValueError("Y must be a contiguous complex128 tensor of shape %s" % (tuple(X.shape),))
+    if len({t.device for t in (X, z, C, Y) if t is not None}) != 1:
+        raise ValueError("the tensors of matrix_resolvent must be on one device")
+    nbytes = X.numel() * X.element_size()
+    if Y.data_ptr() != X.data_ptr() and abs(Y.data_ptr() - X.data_ptr()) < nbytes:
+        raise ValueError("Y overlaps X without being X")
+    return B, M, n_z
+
+
+def _matrix_resolvent(X, z, C, mode, Y):
+    B, M, n_z = check_matrix_resolvent(X, z, C, mode, Y)
+    if B == 0 or n_z == 0:
+        return
+    with torch.cuda.device(Y.device):
+        _lib.check(_lib.load().mx_matrix_resolvent(_ptr(X), B, M, n_z, _ptr(z), _ptr(C), int(mode), _ptr(Y), _stream(Y)),
+                   "mx_matrix_resolvent")
+
+
 _library.impl("project_data", _project_data, "CUDA")
 _library.impl("alpha_sweep", _alpha_sweep, "CUDA")
 _library.impl("analyze", _analyze, "CUDA")
 _library.impl("poorman_models", _poorman_models, "CUDA")
 _library.impl("hilbert_table", _hilbert_table, "CUDA")
 _library.impl("hilbert_apply", _hilbert_apply, "CUDA")
+_library.impl("matrix_resolvent", _matrix_resolvent, "CUDA")
 
 project_data = torch.ops.maxent_b200.project_data
 alpha_sweep = torch.ops.maxent_b200.alpha_sweep
@@ -229,4 +269,6 @@ analyze = torch.ops.maxent_b200.analyze
 poorman_models = torch.ops.maxent_b200.poorman_models
 hilbert_table = torch.ops.maxent_b200.hilbert_table
 hilbert_apply = torch.ops.maxent_b200.hilbert_apply
-OPERATORS = ("project_data", "alpha_sweep", "analyze", "poorman_models", "hilbert_table", "hilbert_apply")
+matrix_resolvent = torch.ops.maxent_b200.matrix_resolvent
+OPERATORS = ("project_data", "alpha_sweep", "analyze", "poorman_models", "hilbert_table", "hilbert_apply",
+             "matrix_resolvent")

@@ -10,12 +10,15 @@ FP64 tensor cores (``mx_hilbert_apply``), with the self-energy algebra of the co
 ``BatchedSigmaContinuator`` is the array-based counterpart of the reference's ``DirectSigmaContinuator`` and
 ``InversionSigmaContinuator`` (python/sigma_continuator.py) for a batch of scalar self-energies Sigma_b(i omega_n):
 auxiliary Green function, batched MaxEnt continuation on the Matsubara axis (``BatchedTauMaxEnt.set_G_iw_data``) and
-Sigma_b(w + i eta) from the analyzer's A_aux without a trip to the host.
+Sigma_b(w + i eta) from the analyzer's A_aux without a trip to the host.  With a matrix worker (``BatchedElementwiseMaxEnt``
+or ``BatchedPoormanMaxEnt``) it continues matrix-valued self-energies Sigma_b(i omega_n)[M, M] by inversion: the two
+matrix inversions run on the device (``mx_matrix_resolvent``), the continuation element by element in between.
 """
 import numpy as np
 
 from . import _lib
 from .batched import ANALYZER_NAMES, BatchedTauMaxEnt
+from .batched_matrix import BatchedElementwiseMaxEnt
 
 _TABLE_CACHE = {}
 _TABLE_CACHE_SIZE = 4
@@ -150,7 +153,11 @@ class BatchedSigmaContinuator(object):
     ``BatchedMaxEntResult``; ``sigma_w(w, eta)`` maps the analyzer's A_aux(omega) back to Sigma_b(w + i eta) on the
     device.  A_aux is used as the continuation returns it: it is NOT renormalised before the transform.
 
-    Matrix-valued self-energies (off-diagonal elements) and covariance matrices of Matsubara data are not supported."""
+    Matrix-valued self-energies S_iw[B, M, M, n_iw] (M <= 8) need a matrix worker, ``maxent=BatchedElementwiseMaxEnt(...)``
+    or ``BatchedPoormanMaxEnt(...)``, and ``method='inversion'``: G_aux(i w) = ((i w + C) 1 - Sigma(i w))^-1 per matrix,
+    element-wise continuation of G_aux, and Sigma(z) = (z + C) 1 - G_aux(z)^-1 with G_aux(z) = T(A_aux') + i T(A_aux'')
+    assembled from the element spectra; ``run()`` returns a ``BatchedMatrixMaxEntResult`` and ``sigma_w`` [B, M, M, n_w].
+    Covariance matrices of Matsubara data are not supported."""
 
     def __init__(self, method="inversion", constant_shift=0.0, sigma_inf=None, norm=None, n_tail=None, maxent=None):
         if method not in ("inversion", "direct"):
@@ -167,19 +174,23 @@ class BatchedSigmaContinuator(object):
         self.G_aux_iw = None
         self.result = None
         self._scale = self._shift = None
+        self._matrix = False
 
     def set_S_iw_data(self, iomega, S_iw):
-        """iomega[n_iw] (real Matsubara frequencies), S_iw[B, n_iw] (complex, numpy or tensor): builds G_aux_iw and
-        hands it to ``self.maxent``."""
+        """iomega[n_iw] (real Matsubara frequencies), S_iw[B, n_iw] (complex, numpy or tensor; [B, M, M, n_iw] with a
+        matrix worker): builds G_aux_iw and hands it to ``self.maxent``."""
         nu = np.array(iomega, dtype=np.float64)
         if nu.ndim != 1 or len(nu) < 1:
             raise ValueError("iomega must be a vector of Matsubara frequencies")
+        if isinstance(self.maxent, BatchedElementwiseMaxEnt):
+            return self._set_matrix_S_iw(nu, S_iw)
         S = S_iw.detach().cpu().numpy() if hasattr(S_iw, "detach") else np.asarray(S_iw)
         if S.ndim == 1:
             S = S[None, :]
         if S.ndim != 2:
-            raise NotImplementedError("matrix-valued self-energies (off-diagonal elements) are not supported: pass "
-                                      "scalar self-energies S_iw[B, n_iw]")
+            raise NotImplementedError("matrix-valued self-energies S_iw[B, M, M, n_iw] need a matrix worker: "
+                                      "BatchedSigmaContinuator(maxent=BatchedElementwiseMaxEnt(...)) or "
+                                      "maxent=BatchedPoormanMaxEnt(...); the default worker takes S_iw[B, n_iw]")
         if S.shape[1] != len(nu):
             raise ValueError("iomega and S_iw don't have the same length (%d, %d)" % (len(nu), S.shape[1]))
         S = S.astype(np.complex128)
@@ -200,10 +211,46 @@ class BatchedSigmaContinuator(object):
         self.iomega = nu
         self.G_aux_iw = G_aux
         self.result = None
+        self._matrix = False
+        self.maxent.set_G_iw_data(nu, G_aux)
+
+    def _set_matrix_S_iw(self, nu, S_iw):
+        """Matrix-valued Sigma with a matrix worker: G_aux_iw = ((i nu + C) 1 - Sigma)^-1 on the device
+        (mx_matrix_resolvent mode 0), kept there as a complex128 tensor [B, M, M, n_iw]."""
+        import torch
+        from . import ops
+        S = S_iw if torch.is_tensor(S_iw) else np.asarray(S_iw)
+        shape = tuple(S.shape)
+        if len(shape) != 4:
+            raise ValueError("a matrix worker continues matrix-valued self-energies S_iw[B, M, M, n_iw], got shape %s"
+                             % (shape,))
+        if self.method != "inversion":
+            raise NotImplementedError("method='direct' is not supported for matrix-valued self-energies (it needs a matrix "
+                                      "normalisation of Sigma - Sigma_inf): use method='inversion'")
+        B, M, n_iw = shape[0], shape[1], shape[3]
+        if shape[2] != M:
+            raise NotImplementedError("non-square blocks S_iw[B, %d, %d, n_iw] are not supported" % (shape[1], shape[2]))
+        if not 1 <= M <= _lib.MX_MAX_MATRIX:
+            raise NotImplementedError("blocks of M = %d orbitals are not supported (1 <= M <= %d)" % (M, _lib.MX_MAX_MATRIX))
+        if n_iw != len(nu):
+            raise ValueError("iomega and S_iw don't have the same length (%d, %d)" % (len(nu), n_iw))
+        C = _per_spectrum(self.constant_shift, B, "constant_shift")
+        dev = _device(self.maxent.maxent_diagonal.device)
+        X = (S if torch.is_tensor(S) else torch.from_numpy(np.ascontiguousarray(S)))
+        X = X.to(device=dev, dtype=torch.complex128).contiguous()
+        z = torch.complex(torch.zeros(n_iw, dtype=torch.float64), torch.from_numpy(nu)).to(dev)
+        G_aux = torch.empty_like(X)
+        with torch.cuda.device(dev):
+            ops.matrix_resolvent(X, z, torch.as_tensor(C, device=dev), 0, G_aux)
+        self.iomega = nu
+        self.G_aux_iw = G_aux
+        self.result = None
+        self._scale, self._shift, self._matrix = None, C, True
         self.maxent.set_G_iw_data(nu, G_aux)
 
     def run(self):
-        """The batched continuation of G_aux_iw: a BatchedMaxEntResult (A_out = A_aux of every analyzer)."""
+        """The batched continuation of G_aux_iw: a BatchedMaxEntResult (A_out = A_aux of every analyzer), a
+        BatchedMatrixMaxEntResult with a matrix worker."""
         if self.G_aux_iw is None:
             raise Exception("no data: call set_S_iw_data")
         self.result = self.maxent.run()
@@ -212,13 +259,18 @@ class BatchedSigmaContinuator(object):
     def sigma_w(self, w, eta, analyzer="LineFitAnalyzer"):
         """Sigma_b(w + i eta), complex128 tensor [B, n_w] on the device, from the analyzer's A_aux(omega) of ``run()``
         (read from the device result in place).  Spectra without that analyzer's pick (alpha_index -1: analyzer not
-        available, or G_aux below G_threshold) are NaN rows."""
+        available, or G_aux below G_threshold) are NaN rows.
+
+        Matrix-valued Sigma: [B, M, M, n_w].  A_aux of every element is the result's A_out (zero below G_threshold,
+        NaN without a pick), assembled on the device; a matrix with a NaN element is NaN at every frequency."""
         import torch
         if self.result is None:
             raise Exception("call run() first")
         if analyzer not in ANALYZER_NAMES:
             raise ValueError("unknown analyzer %r (one of %s)" % (analyzer, ", ".join(ANALYZER_NAMES)))
         slot = ANALYZER_NAMES.index(analyzer)
+        if self._matrix:
+            return self._matrix_sigma_w(w, _eta(eta), slot)
         dev = self.result.device
         eta = _eta(eta)
         M, w_d = hilbert_table(np.asarray(self.result.omega), w, eta, device=dev.A_out.device)
@@ -227,3 +279,35 @@ class BatchedSigmaContinuator(object):
         mode = 2 if self.method == "inversion" else 1
         out = _apply(A, M, w_d, eta, mode, put(self._scale), put(self._shift))
         return out.masked_fill_((dev.alpha_index[:, slot] < 0)[:, None], complex(float("nan"), float("nan")))
+
+    def _matrix_sigma_w(self, w, eta, slot):
+        res = self.result
+        return matrix_sigma_w(res.A_out_device(slot), np.asarray(res.omega), w, eta, self._shift)
+
+
+def matrix_sigma_w(A, omega, w, eta, shift=None):
+    """Sigma_b(z_k) = (z_k + C_b) 1 - G_b(z_k)^-1 at z_k = w_k + i eta, complex128 [B, M, M, n_w] on A's device, for
+    matrix spectra A[B, M, M, n_omega] (real elements) or [B, M, M, 2, n_omega] (real and imaginary part of Hermitian
+    A = A' + i A'') given as float64 device tensors on the mesh ``omega``: G(z) = T(A') + i T(A''), T the retarded
+    transform of every part (mx_hilbert_apply mode 0), and the inverse per matrix and frequency (mx_matrix_resolvent
+    mode 1, in place).  ``shift`` C is None or [B].  A matrix with a NaN element is NaN at every frequency."""
+    import torch
+    from . import ops
+    om, eta = _mesh(omega), _eta(eta)
+    B, M, n_omega = int(A.shape[0]), int(A.shape[1]), int(A.shape[-1])
+    if A.dim() not in (4, 5) or int(A.shape[2]) != M or n_omega != len(om) or (A.dim() == 5 and int(A.shape[3]) != 2):
+        raise ValueError("A must be [B, M, M, (2,) %d], got %s" % (len(om), tuple(A.shape)))
+    M_d, w_d = hilbert_table(om, w, eta, device=A.device)
+    n_w = int(M_d.shape[0])
+    T = _apply(_rows(A.reshape(-1, n_omega), n_omega, M_d.device), M_d, w_d, eta, 0)
+    if A.dim() == 5:
+        T = torch.view_as_real(T).reshape(B, M, M, 2, n_w, 2)
+        X = torch.complex(T[:, :, :, 0, :, 0] - T[:, :, :, 1, :, 1], T[:, :, :, 0, :, 1] + T[:, :, :, 1, :, 0])
+        X = X.contiguous()
+    else:
+        X = T.reshape(B, M, M, n_w)
+    z = torch.complex(w_d, torch.full_like(w_d, eta))
+    C = None if shift is None else torch.as_tensor(_per_spectrum(shift, B, "shift"), device=X.device)
+    with torch.cuda.device(X.device):
+        ops.matrix_resolvent(X, z, C, 1, X)
+    return X
